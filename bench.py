@@ -2,6 +2,7 @@
 """bench.py — TT-SVD GElements/s on B200 (BASELINE.json metric), one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape 64,64,64,64,64] [--rank 32]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 A "step" = one tnb_ttsvd_batch call per GPU: the complete TT-SVD (tn.Tensor(X[B, ...], ranks_tt=r, batch=True)) of
@@ -40,11 +41,35 @@ def parse():
                     help="independent tensors per GPU and step, decomposed by ONE tnb_ttsvd_batch call (the library keeps "
                          "them in flight on internal streams: the latency-bound eigen chains of one tensor run beside the "
                          "bandwidth-bound Gram/projection kernels of another)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the TT cores of the last step as DIR/tensor<i>_core<k>.npy "
+                         "(inputs are seeded, so two builds run with the same arguments can be compared file by file)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 METRIC = "TT-SVD GElements/s"
 _json_out = sys.stdout  # replaced in __main__ by a duplicate of the real fd 1 (everything else goes to stderr)
+DUMP_BUDGET_BYTES = 64 << 20  # all files written by one process's --dump-outputs together
+
+
+def dump_outputs(directory, arrays, budget=DUMP_BUDGET_BYTES):
+    """Write `arrays` (name -> torch tensor or NumPy array, float32 or float64) as DIR/<name>.npy.  When they are larger
+    than `budget` in all, each array is cut to the same fixed, seeded sample of its flattened elements, so that two runs
+    with the same arguments still write comparable files."""
+    import numpy as np
+
+    host = {n: a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a) for n, a in arrays.items()}
+    total = sum(x.nbytes for x in host.values())
+    keep = min(1.0, budget / total) if total else 1.0
+    os.makedirs(directory, exist_ok=True)
+    for name, x in host.items():
+        if keep < 1.0:
+            flat = x.reshape(-1)
+            x = flat[np.sort(np.random.default_rng(0).choice(flat.size, int(flat.size * keep), replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), x)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -168,8 +193,10 @@ def run_reference(args):
     times = []
     for i in range(args.steps):
         X = arm.make_input(i)
-        dt, _ = arm.step(X)
+        dt, cores = arm.step(X)
         times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"tensor0_core{k}": c for k, c in enumerate(cores)})
     tot = sum(times)
     value = arm.n * args.steps / tot / 1e9
     out = {
@@ -353,6 +380,11 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_total = float(t.item())
     ms_step = ms_total / args.steps
+    if args.dump_outputs:
+        # every rank writes its own tensors under their global batch index, within its share of the budget
+        dump_outputs(args.dump_outputs, {f"tensor{rank_id * PB + b}_core{k}": c
+                                         for b, tcores in enumerate(cores_list) for k, c in enumerate(tcores)},
+                     budget=DUMP_BUDGET_BYTES // world)
     value = world * PB * numel / (ms_step * 1e-3) / 1e9
     cores = cores_list[0]
     ranks = [1] + [int(c.shape[2]) for c in cores]
