@@ -1,5 +1,5 @@
-"""A/B of the in-flight batch schedule (tnb_ttsvd_batch): prints ms per tensor for the 64^5 / r=32 workload.
-Environment switches read by the library: TNB_BATCH_ORDER=phase|wave, TNB_NO_GATE=1.  Usage: batch_exp.py [inflight] [reserve]"""
+"""Timing of the in-flight batch (tnb_ttsvd_batch): prints ms per tensor for the 64^5 / r=32 workload with `inflight`
+tensors in flight and `reserve` SMs left free by the whole-GPU kernels.  Usage: batch_exp.py [inflight] [reserve]"""
 import sys
 
 import torch

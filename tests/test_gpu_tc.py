@@ -127,11 +127,9 @@ def test_sweep_uses_resident_filter():
 
 
 @pytest.mark.parametrize("name", ["twin32x5_r32_f32", "randn64x4_r32_f32"])
-@pytest.mark.parametrize("narrow", [False, True])
-def test_concurrent_flag_same_result(name, narrow, monkeypatch):
+def test_concurrent_flag_same_result(name):
     """TNB_FLAG_CONCURRENT only changes scheduling (whole-GPU kernels chained across streams and sized to leave
-    the reserved SMs free, no resident filter kernel): ranks and error must match the golden vectors just the same.
-    TNB_NARROW additionally routes the filter products through the one-CTA-per-tile direct-epilogue form."""
+    the reserved SMs free, no resident filter kernel): ranks and error must match the golden vectors just the same."""
     import os
 
     import numpy as np
@@ -139,8 +137,6 @@ def test_concurrent_flag_same_result(name, narrow, monkeypatch):
     from oracle import cases
     from tntorch_b200 import ops
 
-    if narrow:
-        monkeypatch.setenv("TNB_NARROW", "1")
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ttsvd.npz"))
     spec = cases.TTSVD_CASES[name]
     X = cases.make_dense(spec)

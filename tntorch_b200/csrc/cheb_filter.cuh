@@ -362,7 +362,6 @@ inline int cheb_filter_f32(const float* G, int n, int b, float* const bufs[3], i
     cudaGetLastError();
     fail(TNB_ERR_UNSUPPORTED, "resident filter launch refused: %s (n=%d b=%d smem=%zu dsmem=%d, max active clusters %d)",
          cudaGetErrorString(e), n, b, smem, p.dsmem, max_clusters);
-    if (getenv("TNB_DEBUG")) fprintf(stderr, "tnb200: %s\n", last_error_ref().c_str());
     ds.refused |= 1u << (n / 256);
     return TNB_ERR_UNSUPPORTED;
   }

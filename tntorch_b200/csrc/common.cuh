@@ -158,11 +158,11 @@ inline int usable_sms() {
 
 // TNB_FLAG_CONCURRENT: the bandwidth-bound whole-GPU kernels (tensor-core Gram, projection) of the decompositions in
 // flight are chained across their streams, one at a time, each sized to usable_sms(): the reserved SMs then stay free
-// for the latency-bound eigen chains of the OTHER decompositions (one-CTA Jacobi / Cholesky kernels, narrow
+// for the latency-bound eigen chains of the OTHER decompositions (one-CTA Jacobi / Cholesky kernels, small
 // products), which would otherwise queue behind — or steal an SM from and double the time of — a one-wave kernel.
 class BigKernelGate {
  public:
-  BigKernelGate(cudaStream_t st, bool enabled) : st_(st), on_(enabled && !disabled()), dev_(enabled ? current_device_index() : 0) {
+  BigKernelGate(cudaStream_t st, bool enabled) : st_(st), on_(enabled), dev_(enabled ? current_device_index() : 0) {
     if (!on_) return;
     mu().lock();
     cudaEvent_t& e = ev();
@@ -182,7 +182,6 @@ class BigKernelGate {
   BigKernelGate& operator=(const BigKernelGate&) = delete;
 
  private:
-  static bool disabled() { static const bool d = getenv("TNB_NO_GATE") != nullptr; return d; }  // A/B switch
   // one gate (mutex + event) per device: big kernels of different GPUs never wait on each other
   std::mutex& mu() { static std::mutex m[TNB_MAX_DEVICES]; return m[dev_]; }
   cudaEvent_t& ev() { static cudaEvent_t e[TNB_MAX_DEVICES] = {}; return e[dev_]; }

@@ -39,7 +39,6 @@ struct ChfsiWork {
   void* partial;            // split-K scratch, partial_bytes
   size_t partial_bytes;
   bool use_tc = false;      // filter products on the tcgen05 kernel (fp32 blocks only)
-  bool narrow = false;      // products on one CTA per output tile with a direct epilogue (opt-in, TNB_NARROW; measured slower)
   bool shared_gpu = false;  // TNB_FLAG_CONCURRENT: other decompositions run beside this one: no resident 128-SM filter kernel
   double *S, *lam, *Q, *d;  // b*b, b, b*b, b
   double* jscratch;         // jacobi_scratch_doubles(b)
@@ -85,7 +84,7 @@ inline int chfsi_apply(const TB* G, int n, int b, const TB* Yin, const TB* Xin, 
     return atb_tc_f32(reinterpret_cast<const float*>(G), n, n, reinterpret_cast<const float*>(Yin), b,
                       reinterpret_cast<float*>(Yout), b, (float)a, (bc != 0.0 ? reinterpret_cast<const float*>(Yin) : nullptr),
                       b, (float)bc, (g != 0.0 ? reinterpret_cast<const float*>(Xin) : nullptr), b, (float)g, w.partial,
-                      w.partial_bytes, st, w.narrow);
+                      w.partial_bytes, st);
   GemmPlan pl = plan_gemm(n, b, n, false);
   return gemm_splitk<TB, TB, TB, TB, TB>(pl, n, b, n, G, n, /*a_kmaj (symmetric: either)*/ false, Yin, b, false,
                                          reinterpret_cast<TB*>(w.partial), Yout, b, (TB)a, (bc != 0.0 ? Yin : nullptr), b,
@@ -224,8 +223,7 @@ inline int eig_topk_chfsi(const TB* G, int n, int k, int b, const double* d_trac
         if (all3[q] != X) bufs[c3++] = all3[q];
     }
     bool fused = false;
-    if (w.use_tc && !w.narrow && !w.shared_gpu && std::is_same<TB, float>::value && m <= CF_MAX_STEPS &&
-        !getenv("TNB_NO_RESIDENT_FILTER")) {
+    if (w.use_tc && !w.shared_gpu && std::is_same<TB, float>::value && m <= CF_MAX_STEPS) {
       // the whole filter as one resident kernel (cheb_filter.cuh); same recurrence, coefficients precomputed
       float fa[CF_MAX_STEPS], fb[CF_MAX_STEPS], fg[CF_MAX_STEPS];
       double sg = sigma1;

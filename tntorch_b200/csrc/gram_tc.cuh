@@ -51,15 +51,6 @@ struct GramTcParams {
   uint32_t desc_sbo;     // bytes between K atoms (4 rows x 128 B)
   int fold;              // > 1: the matrix was viewed as (rows/fold) x (fold*n_orig); G = sum of the diagonal blocks
   int n_orig;
-  // direct epilogue (general A^T B with ksplit == 1): C = alpha * acc + beta * D + gamma * E written by the
-  // epilogue warps, no partial tiles and no finalize kernel.  One CTA per output tile: the narrow form used
-  // when several decompositions share the GPU (few SMs busy per product instead of all of them).
-  int direct;
-  float* C;
-  const float* D;
-  const float* E;
-  int ldc, ldd, lde;
-  float alpha, beta, gamma;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -283,35 +274,7 @@ gram_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__
     const int lane_group = warp_idx & 3;          // TMEM lanes [32*lane_group, +32)
     const int row = lane_group * 32 + lane;       // accumulator row = column (a_col0 + row) of C
     float* out = p.partial + (((size_t)split * p.num_tiles + tile_id) * 128 + row) * (size_t)p.tn;
-    if (p.direct) {
-      const int gi = a_col0 + row;  // output row
-      if (iters > 0) {
-        mbar_wait(tmem_full_bar, 0);
-        tcgen05_fence_after();
-      }
-      for (int c0 = 0; c0 < p.tn; c0 += 32) {
-        uint32_t v[32];
-        if (iters > 0) {
-          tmem_ld_32x32b_x32(tmem_base + ((uint32_t)(lane_group * 32) << 16) + (uint32_t)c0, v);
-          tmem_ld_wait();
-        } else {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) v[i] = 0u;
-        }
-        if (gi < p.m) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            const int gj = b_col0 + c0 + i;
-            if (gj < p.n) {
-              float x = p.alpha * __uint_as_float(v[i]);
-              if (p.D) x += p.beta * p.D[(size_t)gi * p.ldd + gj];
-              if (p.E) x += p.gamma * p.E[(size_t)gi * p.lde + gj];
-              p.C[(size_t)gi * p.ldc + gj] = x;
-            }
-          }
-        }
-      }
-    } else if (iters > 0) {
+    if (iters > 0) {
       mbar_wait(tmem_full_bar, 0);
       tcgen05_fence_after();
       for (int c0 = 0; c0 < p.tn; c0 += 32) {
@@ -446,12 +409,6 @@ inline void gram_tc_plan(int64_t rows, int64_t n, GramTcParams& p, int64_t m_col
   p.desc_sbo = 512;
   p.fold = 1;
   p.n_orig = (int)n;
-  p.direct = 0;
-  p.C = nullptr;
-  p.D = p.E = nullptr;
-  p.ldc = p.ldd = p.lde = 0;
-  p.alpha = 1.f;
-  p.beta = p.gamma = 0.f;
 }
 
 // Narrow matrices (n = 32 or 64) are viewed as (rows/f) x 128, f = 128/n: one full-width 128 x 128 tile with
@@ -558,22 +515,14 @@ inline int encode_rowmajor_f32(CUtensorMap* tmap, const float* ptr, int64_t rows
 
 inline int atb_tc_f32(const float* A, int64_t K, int64_t m, const float* B, int64_t n, float* C, int ldc, float alpha,
                       const float* D, int ldd, float beta, const float* E, int lde, float gamma, void* ws,
-                      size_t ws_bytes, cudaStream_t st, bool narrow = false) {
+                      size_t ws_bytes, cudaStream_t st) {
   if (!tc_path_available()) return fail(TNB_ERR_UNSUPPORTED, "atb_tc: tcgen05/TMA path needs an sm_100 device");
   if (!atb_tc_shape_ok(K, m, n)) return fail(TNB_ERR_UNSUPPORTED, "atb_tc: unsupported shape K=%lld m=%lld n=%lld", (long long)K, (long long)m, (long long)n);
   if (((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(B)) & 15u) != 0)
     return fail(TNB_ERR_INVALID, "atb_tc: operands must be 16-byte aligned");
   GramTcParams p;
   gram_tc_plan(K, n, p, m);
-  if (narrow) {  // one CTA per output tile, epilogue writes C directly
-    p.ksplit = 1;
-    p.iters_per_split = p.iters_total;
-    p.direct = 1;
-    p.C = C; p.ldc = ldc; p.alpha = alpha;
-    p.D = beta != 0.f ? D : nullptr; p.ldd = ldd; p.beta = beta;
-    p.E = gamma != 0.f ? E : nullptr; p.lde = lde; p.gamma = gamma;
-  }
-  const size_t need = narrow ? 0 : (size_t)p.ksplit * p.num_tiles * 128 * p.tn * sizeof(float);
+  const size_t need = (size_t)p.ksplit * p.num_tiles * 128 * p.tn * sizeof(float);
   if (ws_bytes < need) return fail(TNB_ERR_WORKSPACE, "atb_tc: workspace %zu < %zu", ws_bytes, need);
   p.partial = static_cast<float*>(ws);
   CUtensorMap ta, tb;
@@ -584,7 +533,6 @@ inline int atb_tc_f32(const float* A, int64_t K, int64_t m, const float* B, int6
   dim3 grid((unsigned)p.num_tiles, (unsigned)p.ksplit);
   gram_tc_kernel<<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(ta, tb, p);
   TNB_LAUNCH_CHECK();
-  if (narrow) return TNB_OK;
   const int64_t total = m * n;
   atb_tc_finalize_kernel<<<(unsigned)std::min<int64_t>((total + 255) / 256, 4096), 256, 0, st>>>(p, C, ldc, alpha, D, ldd,
                                                                                                  beta, E, lde, gamma);

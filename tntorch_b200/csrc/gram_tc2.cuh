@@ -15,8 +15,13 @@
 
 namespace tnb {
 
-constexpr int TC2_STAGE_BYTES = 8 * TC_BOX_BYTES;  // A_r: 4 boxes, B_r: 4 boxes (32 KB)
-constexpr int TC2_STAGES = 6;
+// KC rows of C per pipeline stage in 8 KB TMA boxes, 3 stages: 64 measured 21 % faster than 32-row boxes with 6 stages
+// on the 262144 x 2048 Gram (half as many TMA instructions and barrier round trips per byte for the single producer /
+// issuer threads; profiles/r02_gram_tc2_depth.md)
+constexpr int TC2_KC = 64;
+constexpr int TC2_BOX_BYTES = TC2_KC * 128;          // one TMA box: 32 fp32 columns x KC rows
+constexpr int TC2_STAGE_BYTES = 8 * TC2_BOX_BYTES;   // A_r: 4 boxes, B_r: 4 boxes (64 KB)
+constexpr int TC2_STAGES = 3;
 constexpr int TC2_SMEM_BYTES = TC2_STAGES * TC2_STAGE_BYTES + 1024 + 256;
 
 struct GramTc2Params {
@@ -66,14 +71,8 @@ __device__ __forceinline__ void tcgen05_mma_tf32_pair(uint32_t tmem_d, uint64_t 
       : "memory");
 }
 
-// KC rows of C per pipeline stage (32: 4 KB TMA boxes, 6 stages; 64: 8 KB boxes, 3 stages — half as many TMA instructions
-// and barrier round trips per byte for the single producer / issuer threads; A/B in profiles/r02_gram_tc2_depth.md)
-template <int KC, int STAGES>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
-gram_tc2_kernel_t(const __grid_constant__ CUtensorMap tmap, const GramTc2Params p) {
-  constexpr int BOX_BYTES = KC * 128;
-  constexpr int TC2_STAGE_BYTES = 8 * BOX_BYTES;
-  constexpr int TC2_STAGES = STAGES;
+gram_tc2_kernel(const __grid_constant__ CUtensorMap tmap, const GramTc2Params p) {
   extern __shared__ unsigned char tc2_smem_raw[];
   const uint32_t raw_addr = smem_u32(tc2_smem_raw);
   const uint32_t pad = (1024u - (raw_addr & 1023u)) & 1023u;
@@ -127,12 +126,12 @@ gram_tc2_kernel_t(const __grid_constant__ CUtensorMap tmap, const GramTc2Params 
       for (int64_t it = 0; it < iters; ++it) {
         mbar_wait(&empty_bar[stage], phase ^ 1u);
         unsigned char* sb = stage_base + stage * TC2_STAGE_BYTES;
-        if (cta_rank == 0) mbar_expect_tx(&full_bar[stage], 2u * (uint32_t)nbox * BOX_BYTES);  // bytes of BOTH CTAs
-        const int row0 = (int)((it_begin + it) * KC);
-        for (int j = 0; j < 4; ++j) tma_load_2d_pair(sb + j * BOX_BYTES, &tmap, &full_bar[stage], b_col0 + 32 * j, row0);
+        if (cta_rank == 0) mbar_expect_tx(&full_bar[stage], 2u * (uint32_t)nbox * TC2_BOX_BYTES);  // bytes of BOTH CTAs
+        const int row0 = (int)((it_begin + it) * TC2_KC);
+        for (int j = 0; j < 4; ++j) tma_load_2d_pair(sb + j * TC2_BOX_BYTES, &tmap, &full_bar[stage], b_col0 + 32 * j, row0);
         if (!diag)
           for (int j = 0; j < 4; ++j)
-            tma_load_2d_pair(sb + (4 + j) * BOX_BYTES, &tmap, &full_bar[stage], a_col0 + 32 * j, row0);
+            tma_load_2d_pair(sb + (4 + j) * TC2_BOX_BYTES, &tmap, &full_bar[stage], a_col0 + 32 * j, row0);
         if (++stage == TC2_STAGES) { stage = 0; phase ^= 1u; }
       }
     }
@@ -147,11 +146,11 @@ gram_tc2_kernel_t(const __grid_constant__ CUtensorMap tmap, const GramTc2Params 
         tcgen05_fence_after();
         const uint32_t sb = smem_u32(stage_base + stage * TC2_STAGE_BYTES);
         const uint32_t b_addr = sb;
-        const uint32_t a_addr = diag ? sb : sb + 4u * BOX_BYTES;
+        const uint32_t a_addr = diag ? sb : sb + 4u * TC2_BOX_BYTES;
 #pragma unroll
-        for (int ks = 0; ks < KC / 8; ++ks) {
-          const uint64_t adesc = make_mn_major_desc(a_addr + ks * 1024u, BOX_BYTES, 512u, 1u);
-          const uint64_t bdesc = make_mn_major_desc(b_addr + ks * 1024u, BOX_BYTES, 512u, 1u);
+        for (int ks = 0; ks < TC2_KC / 8; ++ks) {
+          const uint64_t adesc = make_mn_major_desc(a_addr + ks * 1024u, TC2_BOX_BYTES, 512u, 1u);
+          const uint64_t bdesc = make_mn_major_desc(b_addr + ks * 1024u, TC2_BOX_BYTES, 512u, 1u);
           tcgen05_mma_tf32_pair(tmem_base, adesc, bdesc, idesc, (it > 0 || ks > 0) ? 1u : 0u);
         }
         tcgen05_commit_pair(&empty_bar[stage]);  // frees the stage in both CTAs
@@ -208,18 +207,12 @@ __global__ void gram_tc2_finalize_kernel(const GramTc2Params p, double* __restri
 
 inline bool gram_tc2_shape_ok(int64_t rows, int64_t n) { return n >= 512 && gram_tc_shape_ok(rows, n); }
 
-inline int gram_tc2_kc() {
-  // 64 measured 21 % faster than 32 on the 262144 x 2048 Gram (profiles/r02_gram_tc2_depth.md); TNB_TC2_KC=32 switches back
-  static const int kc = (getenv("TNB_TC2_KC") && atoi(getenv("TNB_TC2_KC")) == 32) ? 32 : 64;
-  return kc;
-}
 inline void gram_tc2_plan(int64_t rows, int64_t n, GramTc2Params& p) {
   p.rows = rows;
   p.n = (int)n;
   p.nb = (int)((n + 255) / 256);
   p.num_tiles = p.nb * (p.nb + 1) / 2;
-  const int kc = gram_tc2_kc();
-  p.iters_total = (rows + kc - 1) / kc;
+  p.iters_total = (rows + TC2_KC - 1) / TC2_KC;
   const int sms = usable_sms();
   int64_t ks = (sms / 2) / p.num_tiles;
   if (ks < 1) ks = 1;
@@ -245,18 +238,11 @@ inline int gram_tc2_f32(const float* A, int64_t rows, int64_t n, double* G, floa
   if (ws_bytes < need) return fail(TNB_ERR_WORKSPACE, "gram_tc2: workspace %zu < %zu", ws_bytes, need);
   p.partial = static_cast<float*>(ws);
   CUtensorMap tmap;
-  const int kc = gram_tc2_kc();
-  TNB_TRY(encode_rowmajor_f32(&tmap, A, rows, n, kc));
-  static PerDeviceFlag attr_done[2];
+  TNB_TRY(encode_rowmajor_f32(&tmap, A, rows, n, TC2_KC));
+  static PerDeviceFlag attr_done;
+  TNB_CUDA(ensure_dyn_smem(attr_done, gram_tc2_kernel, TC2_SMEM_BYTES));
   dim3 grid((unsigned)(2 * p.num_tiles), (unsigned)p.ksplit);
-  if (kc == 64) {
-    constexpr int SM = 3 * 8 * 64 * 128 + 1024 + 256;
-    TNB_CUDA(ensure_dyn_smem(attr_done[1], gram_tc2_kernel_t<64, 3>, SM));
-    gram_tc2_kernel_t<64, 3><<<grid, TC_THREADS, SM, st>>>(tmap, p);
-  } else {
-    TNB_CUDA(ensure_dyn_smem(attr_done[0], gram_tc2_kernel_t<32, 6>, TC2_SMEM_BYTES));
-    gram_tc2_kernel_t<32, 6><<<grid, TC_THREADS, TC2_SMEM_BYTES, st>>>(tmap, p);
-  }
+  gram_tc2_kernel<<<grid, TC_THREADS, TC2_SMEM_BYTES, st>>>(tmap, p);
   TNB_LAUNCH_CHECK();
   const int64_t total = n * n;
   gram_tc2_finalize_kernel<<<(unsigned)std::min<int64_t>((total + 255) / 256, 4096), 256, 0, st>>>(p, G, Gf);

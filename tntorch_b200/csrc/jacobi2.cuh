@@ -359,12 +359,10 @@ inline int jacobi2_threads(int n) {
 // Same contract as jacobi_eigh (jacobi.cuh); falls back to it outside the shared-memory envelope.
 inline int jacobi2_eigh(const double* G, int n, int ldg, double* w, double* V, double* scratch, int* info, cudaStream_t st,
                         bool single_precision = false, double loose_tol = 0.0) {
-  static const bool disabled = getenv("TNB_NO_JACOBI2") != nullptr;  // A/B switch (profiling)
-  if (disabled || !jacobi2_ok(n, single_precision)) return jacobi_eigh(G, n, ldg, w, V, scratch, info, st, single_precision, loose_tol);
+  if (!jacobi2_ok(n, single_precision)) return jacobi_eigh(G, n, ldg, w, V, scratch, info, st, single_precision, loose_tol);
   const int max_sweeps = 30;
   static PerDeviceFlag attr_done[3];
-  static const bool no_mixed = getenv("TNB_NO_MIXED_JACOBI") != nullptr;  // A/B switch
-  if (!single_precision && !no_mixed && n <= JAC2_MIXED_MAX_N && n >= 8) {
+  if (!single_precision && n <= JAC2_MIXED_MAX_N && n >= 8) {
     const double tol = loose_tol > 0.0 ? loose_tol : 1e-14;
     const size_t smem = jac2_smem_bytes<double>(n) + jac2_smem_bytes<float>(n);
     TNB_CUDA(ensure_dyn_smem(attr_done[2], jacobi2_mixed_kernel,

@@ -69,8 +69,7 @@ inline int tt_round_impl(ArenaT& ar, bool dry, const T* const* cores_in, const R
   cx.flags = flags;
   cx.allow_tc = false;  // TT cores are small: the generic fp64-accumulating kernels are used throughout
   cx.st = st;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(N - 1)));
-  cx.eps_scaled2 = epsN * epsN;
+  cx.eps_scaled2 = eps_budget2(eps, N);
   cx.sc = ar.template take<SweepScalars>(1);
   if (!dry) {
     cx.h_sc = static_cast<int*>(pinned_scratch(sizeof(SweepScalars)));
@@ -222,10 +221,8 @@ __global__ void or_flag_kernel(const int* src, int* flags, int bit) {
 
 template <typename T>
 inline bool tt_round_spec_eligible(const RoundDims& d, const int32_t* rmax, double eps, uint32_t flags) {
-  static const bool disabled = getenv("TNB_NO_SPECULATE") != nullptr;
-  if (disabled || (flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(d.N - 1)));
-  if (!(epsN * epsN < 1e-20)) return false;
+  if ((flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
+  if (!(eps_budget2(eps, d.N) < 1e-20)) return false;
   for (int k = 0; k < d.N - 1; ++k) {
     if (rmax[k] <= 0) return false;
     if (d.ra[k + 1] != d.rin[k + 1] || d.ra[k] * d.shape[k] < d.rin[k + 1]) return false;  // Cholesky-QR keeps every column
@@ -244,8 +241,7 @@ inline int tt_round_spec_enqueue(ArenaT& ar, bool dry, const T* const* cores_in,
   cx.flags = flags;
   cx.allow_tc = false;
   cx.st = st;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(N - 1)));
-  cx.eps_scaled2 = epsN * epsN;
+  cx.eps_scaled2 = eps_budget2(eps, N);
   cx.sc = ar.template take<SweepScalars>(1);
   cx.d_flags = ar.template take<int>(4);
   cx.d_ranks = ar.template take<int32_t>(N + 1);

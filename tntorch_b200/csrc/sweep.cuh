@@ -44,9 +44,26 @@ inline int project_any(const T* A, int64_t rows, int64_t n, const T* V, int64_t 
   return gemm_direct<T, T, T, T>(rows, r, n, A, n, true, V, r, false, C, r, (T)1, nullptr, 0, (T)0, nullptr, 0, (T)0, st);
 }
 
-inline bool gram_use_pairs(int64_t rows, int64_t n) {
-  static const bool disabled = getenv("TNB_GRAM_TC2") && atoi(getenv("TNB_GRAM_TC2")) == 0;  // A/B switch for profiling
-  return !disabled && gram_tc2_shape_ok(rows, n);
+// The project_tc workspace of a (rows x n) -> (rows x kcap) projection, when that kernel may run for it.
+template <typename T, class ArenaT>
+inline void project_tc_carve(ArenaT& ar, bool allow_tc, int64_t rows, int64_t n, int64_t kcap, void** ws, size_t* bytes) {
+  *ws = nullptr;
+  *bytes = 0;
+  if (allow_tc && std::is_same<T, float>::value && rows >= n && rows >= PROJ_TC_MIN_ROWS && kcap <= PT_MAX_N && n % 4 == 0 &&
+      n >= 32) {
+    *bytes = project_tc_workspace_bytes(n, kcap);
+    *ws = ar.template take<char>(*bytes);
+  }
+}
+
+// Tensor cores are used unless the caller opted out; the sizing pass (dry) cannot ask the device and sizes for them.
+inline bool tc_allowed(uint32_t flags, bool dry) { return !(flags & TNB_FLAG_NO_TENSORCORE) && (dry || tc_path_available()); }
+
+// Squared tail-energy budget of one truncation step: the relative error eps is split evenly over the N - 1 bonds
+// (tensor.py:2039-2051).
+inline double eps_budget2(double eps, int N) {
+  const double epsN = eps / std::max(1.0, std::sqrt((double)(N - 1)));
+  return epsN * epsN;
 }
 
 constexpr int64_t TC_MIN_ROWS = 2048;  // below this the generic fp64-accumulating Gram is used
@@ -89,6 +106,18 @@ inline int make_dims(int ndim, const int64_t* shape, const int32_t* rmax, SweepD
   return TNB_OK;
 }
 
+// Ping-pong carries of the right-to-left sweep (step t writes carry[t & 1] and reads the other), sized by the rank caps.
+template <typename T, class ArenaT>
+inline void carry_carve(ArenaT& ar, const SweepDims& d, T* carry[2]) {
+  size_t carry_elems[2] = {0, 0};
+  for (int mu = d.N - 1, t = 0; mu >= 1; --mu, ++t) {
+    const size_t e = (size_t)d.rows[mu] * (size_t)d.rcap[mu];
+    if (e > carry_elems[t & 1]) carry_elems[t & 1] = e;
+  }
+  carry[0] = ar.template take<T>(carry_elems[0]);
+  carry[1] = ar.template take<T>(carry_elems[1]);
+}
+
 // ---------------------------------------------------------------------------------------------
 // Gram of a (rows x n) row-major matrix on whichever side is smaller, into fp64 G (L x L).
 // ---------------------------------------------------------------------------------------------
@@ -124,7 +153,7 @@ inline int gram_small_side(const T* C, int64_t rows, int64_t n, double* G, float
   if (tall) {
     if (use_tc && w.tc_ws && std::is_same<T, float>::value) {
       if (used_tc) *used_tc = 1;
-      if (gram_use_pairs(rows, n))  // wide Gram: 256 x 256 tiles on CTA pairs
+      if (gram_tc2_shape_ok(rows, n))  // wide Gram: 256 x 256 tiles on CTA pairs
         return gram_tc2_f32(reinterpret_cast<const float*>(C), rows, n, G, Gf, w.tc_ws, w.tc_bytes, st);
       return gram_tc_f32(reinterpret_cast<const float*>(C), rows, n, G, Gf, w.tc_ws, w.tc_bytes, st);
     }
@@ -194,7 +223,6 @@ inline int eig_run(const double* G, const TBk* Gb_in, int64_t L, EigWork<TBk>& e
   if (!e.chfsi) return jacobi2_eigh(G, (int)L, (int)L, e.w, e.V, e.jscratch, e.jinfo, st);
   e.cw.use_tc = allow_tc;
   e.cw.shared_gpu = shared_gpu;
-  e.cw.narrow = shared_gpu && getenv("TNB_NARROW") != nullptr;
   e.k_run = (k_try > 0 && k_try < e.k) ? k_try : e.k;
   e.b_run = chfsi_default_block((int)L, e.k_run);
   if (e.b_run > e.b) e.b_run = e.b;
@@ -279,6 +307,21 @@ struct Prof {
   void mark(cudaStream_t st) {
     if (on) cudaEventRecord(next(), st);
   }
+  // after the synchronisation that ends the sweep; 4 events per step: start, after Gram, after eigen+rank, after
+  // factor/projection
+  void report(SweepInfo* info) const {
+    const int steps = used / 4;
+    info->nsteps = steps;
+    for (int t = 0; t < steps && t < 8; ++t) {
+      float a = 0, b = 0, c = 0;
+      cudaEventElapsedTime(&a, ev[4 * t], ev[4 * t + 1]);
+      cudaEventElapsedTime(&b, ev[4 * t + 1], ev[4 * t + 2]);
+      cudaEventElapsedTime(&c, ev[4 * t + 2], ev[4 * t + 3]);
+      info->gram_ms[t] = a;
+      info->eig_ms[t] = b;
+      info->factor_ms[t] = c;
+    }
+  }
   static Prof& get() {
     static thread_local Prof p;
     return p;
@@ -298,6 +341,30 @@ struct StepCtx {
   int* d_flags = nullptr;       // device flags raised by spec_check_kernel / cd_finish_kernel
   int32_t* d_ranks = nullptr;   // device copy of the ranks the rule chose, [N + 1]
 };
+
+// The two factors of a truncation step from the leading eigenpairs (w, V) of the Gram matrix on the smaller side of C:
+// core (rank x n) and Cn (rows x rank) with C ~= Cn * core.  fac is (L x rank) scratch.
+template <typename T>
+inline int split_factors(const T* C, int64_t rows, int64_t n, const double* w, const double* V, int ldv, int64_t rank, T* fac,
+                         void* ptc_ws, size_t ptc_bytes, bool concurrent, T* core, T* Cn, cudaStream_t st) {
+  if (rows >= n) {
+    // core = V_r^T (rank x n);  Cn = C V_r
+    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(V, ldv, (int)n, (int)rank, w, core, 0, 1);
+    TNB_LAUNCH_CHECK();
+    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(V, ldv, (int)n, (int)rank, w, fac, 0, 0);
+    TNB_LAUNCH_CHECK();
+    BigKernelGate gate(st, concurrent && rows >= PROJ_TC_MIN_ROWS);
+    return project_any<T>(C, rows, n, fac, rank, Cn, st, ptc_ws, ptc_bytes);
+  }
+  // core = diag(1/s) U_r^T C (rank x n);  Cn = U_r diag(s)
+  scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(V, ldv, (int)rows, (int)rank, w, fac, 1, 0);
+  TNB_LAUNCH_CHECK();
+  TNB_TRY((gemm_direct<T, T, T, T>(rank, n, rows, fac, rank, false, C, n, false, core, n, (T)1, nullptr, 0, (T)0, nullptr, 0,
+                                   (T)0, st)));
+  scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(V, ldv, (int)rows, (int)rank, w, Cn, 2, 0);
+  TNB_LAUNCH_CHECK();
+  return TNB_OK;
+}
 
 template <typename T, class ArenaT>
 inline int truncate_step(ArenaT& ar, bool dry, const StepCtx& cx, const T* C, int64_t rows, int64_t n, int64_t rank_cap,
@@ -321,13 +388,9 @@ inline int truncate_step(ArenaT& ar, bool dry, const StepCtx& cx, const T* C, in
   TNB_TRY(eig_carve<TBk>(ar, L, kcap, have_rmax, ew));
   if (ew.chfsi && std::is_same<TBk, float>::value) Gf = reinterpret_cast<float*>(ew.Gb);
   T* fac = ar.template take<T>((size_t)L * (size_t)kcap);  // V_r or U_r/s
-  void* ptc_ws = nullptr;
-  size_t ptc_bytes = 0;
-  if (cx.allow_tc && std::is_same<T, float>::value && tall && rows >= PROJ_TC_MIN_ROWS && kcap <= PT_MAX_N && n % 4 == 0 &&
-      n >= 32) {
-    ptc_bytes = project_tc_workspace_bytes(n, kcap);
-    ptc_ws = ar.template take<char>(ptc_bytes);
-  }
+  void* ptc_ws;
+  size_t ptc_bytes;
+  project_tc_carve<T>(ar, cx.allow_tc, rows, n, kcap, &ptc_ws, &ptc_bytes);
   if (dry) return TNB_OK;
   if (!ar.ok) return fail(TNB_ERR_WORKSPACE, "workspace too small (need > %zu bytes)", ar.off);
   Prof& prof = Prof::get();
@@ -370,24 +433,8 @@ inline int truncate_step(ArenaT& ar, bool dry, const StepCtx& cx, const T* C, in
     TNB_LAUNCH_CHECK();
     fill_kernel<T><<<grid_for(rows), 256, 0, st>>>(Cn, rows, (T)0);
     TNB_LAUNCH_CHECK();
-  } else if (tall) {
-    // core = V_r^T (rank x n);  Cn = C V_r
-    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(ew.V, ew.ldv, (int)n, (int)rank, ew.w, core, 0, 1);
-    TNB_LAUNCH_CHECK();
-    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(ew.V, ew.ldv, (int)n, (int)rank, ew.w, fac, 0, 0);
-    TNB_LAUNCH_CHECK();
-    {
-      BigKernelGate gate(st, concurrent && rows >= PROJ_TC_MIN_ROWS);
-      TNB_TRY(project_any<T>(C, rows, n, fac, rank, Cn, st, ptc_ws, ptc_bytes));
-    }
   } else {
-    // core = diag(1/s) U_r^T C (rank x n);  Cn = U_r diag(s)
-    scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(ew.V, ew.ldv, (int)rows, (int)rank, ew.w, fac, 1, 0);
-    TNB_LAUNCH_CHECK();
-    TNB_TRY((gemm_direct<T, T, T, T>(rank, n, rows, fac, rank, false, C, n, false, core, n, (T)1, nullptr, 0, (T)0,
-                                     nullptr, 0, (T)0, st)));
-    scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(ew.V, ew.ldv, (int)rows, (int)rank, ew.w, Cn, 2, 0);
-    TNB_LAUNCH_CHECK();
+    TNB_TRY(split_factors<T>(C, rows, n, ew.w, ew.V, ew.ldv, rank, fac, ptc_ws, ptc_bytes, concurrent, core, Cn, st));
   }
   prof.mark(st);
   *rank_out = rank;
@@ -412,9 +459,9 @@ inline bool spec_step_ok(int64_t rows, int64_t n, int64_t rank_cap, bool allow_t
   return chfsi_dev_ok((int)L, chfsi_dev_block((int)L, (int)k));
 }
 
-// The step is split in two enqueue phases so that a batch of tensors can be interleaved phase by phase (all Gram
-// kernels of a step first, then every tensor's eigen chain + projection): the whole-GPU kernels of the batch then run
-// back to back while the latency-bound eigen chains of the other tensors run beside them on their own streams.
+// The step is split in enqueue phases (Gram; the eigen stages one by one; rank rule + projection) so that a batch of
+// tensors can be interleaved phase by phase (ttsvd_batch_impl): the whole-GPU kernels of the batch then run back to back
+// while the latency-bound eigen chains of the other tensors run beside them on their own streams.
 template <typename T>
 struct SpecStep {
   GramWork<T> gw;
@@ -458,13 +505,7 @@ inline void spec_step_carve(ArenaT& ar, const StepCtx& cx, int64_t rows, int64_t
     chfsi_dev_carve<float>(ar, (int)L, s.b, s.cw);
   }
   s.fac = ar.template take<T>((size_t)L * (size_t)s.kcap);
-  s.ptc_ws = nullptr;
-  s.ptc_bytes = 0;
-  if (cx.allow_tc && std::is_same<T, float>::value && tall && rows >= PROJ_TC_MIN_ROWS && s.kcap <= PT_MAX_N && n % 4 == 0 &&
-      n >= 32) {
-    s.ptc_bytes = project_tc_workspace_bytes(n, s.kcap);
-    s.ptc_ws = ar.template take<char>(s.ptc_bytes);
-  }
+  project_tc_carve<T>(ar, cx.allow_tc, rows, n, s.kcap, &s.ptc_ws, &s.ptc_bytes);
 }
 
 // phase 1: Gram + trace
@@ -514,7 +555,6 @@ inline int spec_step_eig_stage(SpecStep<T>& s, int stage) {
 template <typename T>
 inline int spec_step_rest(const StepCtx& cx, const T* C, int64_t rows, int64_t n, int32_t rm, T* core, T* Cn, int mu,
                           SpecStep<T>& s, bool prof_on) {
-  const bool tall = rows >= n;
   const int64_t L = s.L;
   const int batch_mode = (cx.flags & TNB_FLAG_BATCH_MODE) ? 1 : 0;
   cudaStream_t st = cx.st;
@@ -530,24 +570,7 @@ inline int spec_step_rest(const StepCtx& cx, const T* C, int64_t rows, int64_t n
   spec_check_kernel<<<1, 32, 0, st>>>(cx.sc, (int)s.kcap, cx.d_ranks + mu, cx.d_flags);
   TNB_LAUNCH_CHECK();
   if (prof_on) prof.mark(st);
-  const int64_t rank = s.kcap;
-  if (tall) {
-    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(s.V, s.ldv, (int)n, (int)rank, s.w, core, 0, 1);
-    TNB_LAUNCH_CHECK();
-    scale_extract_kernel<T><<<grid_for(n * rank), 256, 0, st>>>(s.V, s.ldv, (int)n, (int)rank, s.w, s.fac, 0, 0);
-    TNB_LAUNCH_CHECK();
-    {
-      BigKernelGate gate(st, concurrent && rows >= PROJ_TC_MIN_ROWS);
-      TNB_TRY(project_any<T>(C, rows, n, s.fac, rank, Cn, st, s.ptc_ws, s.ptc_bytes));
-    }
-  } else {
-    scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(s.V, s.ldv, (int)rows, (int)rank, s.w, s.fac, 1, 0);
-    TNB_LAUNCH_CHECK();
-    TNB_TRY((gemm_direct<T, T, T, T>(rank, n, rows, s.fac, rank, false, C, n, false, core, n, (T)1, nullptr, 0, (T)0,
-                                     nullptr, 0, (T)0, st)));
-    scale_extract_kernel<T><<<grid_for(rows * rank), 256, 0, st>>>(s.V, s.ldv, (int)rows, (int)rank, s.w, Cn, 2, 0);
-    TNB_LAUNCH_CHECK();
-  }
+  TNB_TRY(split_factors<T>(C, rows, n, s.w, s.V, s.ldv, s.kcap, s.fac, s.ptc_ws, s.ptc_bytes, concurrent, core, Cn, st));
   if (prof_on) prof.mark(st);
   return TNB_OK;
 }
@@ -563,11 +586,10 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
   StepCtx cx;
   cx.flags = flags;
   cx.exact_gram = exact_gram;
-  cx.allow_tc = !(flags & TNB_FLAG_NO_TENSORCORE) && (dry || tc_path_available());
+  cx.allow_tc = tc_allowed(flags, dry);
   cx.info = info;
   cx.st = st;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(N - 1)));
-  cx.eps_scaled2 = epsN * epsN;
+  cx.eps_scaled2 = eps_budget2(eps, N);
   cx.sc = ar.template take<SweepScalars>(1);
   Prof& prof = Prof::get();
   prof.on = !dry && (flags & TNB_FLAG_PROFILE);
@@ -586,13 +608,8 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
     }
     return TNB_OK;
   }
-  // carry buffers (ping-pong), sized by the rank caps
-  size_t carry_elems[2] = {0, 0};
-  for (int mu = N - 1, t = 0; mu >= 1; --mu, ++t) {
-    const size_t e = (size_t)d.rows[mu] * (size_t)d.rcap[mu];
-    if (e > carry_elems[t & 1]) carry_elems[t & 1] = e;
-  }
-  T* carry[2] = {ar.template take<T>(carry_elems[0]), ar.template take<T>(carry_elems[1])};
+  T* carry[2];
+  carry_carve<T>(ar, d, carry);
   const T* C = data;
   int64_t r_next = 1;
   size_t peak = ar.off;
@@ -617,19 +634,7 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
     TNB_CUDA(cudaMemcpyAsync(cores + d.slot[0], C, sizeof(T) * (size_t)d.shape[0] * (size_t)r_next,
                              cudaMemcpyDeviceToDevice, st));
     TNB_CUDA(cudaStreamSynchronize(st));
-    if (prof.on && info) {  // 4 events per step: start, after Gram, after eigen+rank, after factor/projection
-      const int steps = prof.used / 4;
-      info->nsteps = steps;
-      for (int t = 0; t < steps && t < 8; ++t) {
-        float a = 0, b = 0, c = 0;
-        cudaEventElapsedTime(&a, prof.ev[4 * t], prof.ev[4 * t + 1]);
-        cudaEventElapsedTime(&b, prof.ev[4 * t + 1], prof.ev[4 * t + 2]);
-        cudaEventElapsedTime(&c, prof.ev[4 * t + 2], prof.ev[4 * t + 3]);
-        info->gram_ms[t] = a;
-        info->eig_ms[t] = b;
-        info->factor_ms[t] = c;
-      }
-    }
+    if (prof.on && info) prof.report(info);
     prof.on = false;
   }
   return TNB_OK;
@@ -640,10 +645,8 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
 // ---------------------------------------------------------------------------------------------
 template <typename T>
 inline bool spec_eligible(const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, bool allow_tc) {
-  static const bool disabled = getenv("TNB_NO_SPECULATE") != nullptr;  // A/B switch (profiling, debugging)
-  if (disabled || (flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(d.N - 1)));
-  if (!(epsN * epsN < 1e-20)) return false;  // an active eps budget decides ranks: host-driven path
+  if ((flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
+  if (!(eps_budget2(eps, d.N) < 1e-20)) return false;  // an active eps budget decides ranks: host-driven path
   for (int mu = d.N - 1; mu >= 1; --mu) {
     if (rmax[mu - 1] <= 0) return false;
     if (!spec_step_ok<T>(d.rows[mu], d.shape[mu] * d.rcap[mu + 1], d.rcap[mu], allow_tc)) return false;
@@ -683,21 +686,14 @@ inline int spec_begin(SpecRun<T, ArenaT>& r, ArenaT& ar, bool dry, const T* data
   r.ar = &ar;
   r.cx = StepCtx();
   r.cx.flags = flags;
-  r.cx.allow_tc = !(flags & TNB_FLAG_NO_TENSORCORE) && (dry || tc_path_available());
+  r.cx.allow_tc = tc_allowed(flags, dry);
   r.cx.info = info;
   r.cx.st = st;
-  const double epsN = eps / std::max(1.0, std::sqrt((double)(N - 1)));
-  r.cx.eps_scaled2 = epsN * epsN;
+  r.cx.eps_scaled2 = eps_budget2(eps, N);
   r.cx.sc = ar.template take<SweepScalars>(1);
   r.cx.d_flags = ar.template take<int>(4);
   r.cx.d_ranks = ar.template take<int32_t>(N + 1);
-  size_t carry_elems[2] = {0, 0};
-  for (int mu = N - 1, t = 0; mu >= 1; --mu, ++t) {
-    const size_t e = (size_t)d.rows[mu] * (size_t)d.rcap[mu];
-    if (e > carry_elems[t & 1]) carry_elems[t & 1] = e;
-  }
-  r.carry[0] = ar.template take<T>(carry_elems[0]);
-  r.carry[1] = ar.template take<T>(carry_elems[1]);
+  carry_carve<T>(ar, d, r.carry);
   r.C = data;
   r.cores = cores;
   r.peak = ar.off;
@@ -804,19 +800,7 @@ inline int ttsvd_spec_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
   TNB_TRY((spec_end<T, ArenaT>(r, d)));
   TNB_CUDA(cudaStreamSynchronize(st));
   spec_collect(hb, d, ranks_host, info, out);
-  if (prof_on && info) {
-    const int steps = prof.used / 4;
-    info->nsteps = steps;
-    for (int t = 0; t < steps && t < 8; ++t) {
-      float a = 0, b = 0, c = 0;
-      cudaEventElapsedTime(&a, prof.ev[4 * t], prof.ev[4 * t + 1]);
-      cudaEventElapsedTime(&b, prof.ev[4 * t + 1], prof.ev[4 * t + 2]);
-      cudaEventElapsedTime(&c, prof.ev[4 * t + 2], prof.ev[4 * t + 3]);
-      info->gram_ms[t] = a;
-      info->eig_ms[t] = b;
-      info->factor_ms[t] = c;
-    }
-  }
+  if (prof_on && info) prof.report(info);
   prof.on = false;
   return TNB_OK;
 }
@@ -825,9 +809,8 @@ inline int ttsvd_spec_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
 template <typename T, class ArenaT>
 inline int ttsvd_impl(ArenaT& ar, bool dry, const T* data, const SweepDims& d, const int32_t* rmax, double eps,
                       uint32_t flags, T* cores, int32_t* ranks_host, SweepInfo* info, cudaStream_t st) {
-  const bool allow_tc = !(flags & TNB_FLAG_NO_TENSORCORE) && (dry || tc_path_available());
   // the sizing pass cannot ask the device what it supports: size for both paths
-  const bool spec = dry ? (d.N >= 2 && rmax != nullptr) : spec_eligible<T>(d, rmax, eps, flags, allow_tc);
+  const bool spec = dry ? (d.N >= 2 && rmax != nullptr) : spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
   const size_t base = ar.off;
   size_t need_spec = 0;
   if (spec) {
@@ -894,8 +877,7 @@ inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflig
                             const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, T* const* cores,
                             int32_t* ranks_host, double* norms_host, int32_t* spec_host, cudaStream_t st) {
   const int N = d.N;
-  const bool allow_tc = !(flags & TNB_FLAG_NO_TENSORCORE) && tc_path_available();
-  const bool spec = batch > 0 && spec_eligible<T>(d, rmax, eps, flags, allow_tc);
+  const bool spec = batch > 0 && spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
   char* ws = static_cast<char*>(workspace);
   if (!spec || inflight < 2 || batch < 2) {  // one at a time through the dispatcher (speculative when eligible)
     for (int i = 0; i < batch; ++i) {
@@ -929,40 +911,17 @@ inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflig
     for (int s = 0; s < g && rc == TNB_OK; ++s)
       rc = spec_begin<T, Arena>(runs[s], arenas[s], false, data[g0 + s], d, eps, bflags, cores[g0 + s], &infos[g0 + s],
                                 pool.st[s], hbs + g0 + s);
-    // Enqueue order (TNB_BATCH_ORDER, measured on B200 with 6 x 64^5 in flight — profiles/r02_batch_schedule.md):
-    //   "stage" (default): step by step; all Gram kernels of a step, then the eigen stages of all tensors INTERLEAVED
-    //            stage by stage (the resident filter kernels of all streams run one after the other, cheb_filter.cuh:
-    //            this way tensor A's Rayleigh-Ritz step is in flight while tensor B's filter runs), then every
-    //            tensor's rank rule + projection;
-    //   "phase": step by step, each tensor's whole eigen chain enqueued at once (chains then queue behind each other);
-    //   "wave":  a diagonal wavefront — in wave w tensor s is at step w - s.
-    static const char* order_env = getenv("TNB_BATCH_ORDER");
-    const bool order_phase = order_env && !strcmp(order_env, "phase");
-    const bool order_wave = order_env && !strcmp(order_env, "wave");
-    const int steps = N - 1;
-    if (order_wave) {
-      for (int w = 0; w < steps + g - 1 && rc == TNB_OK; ++w) {
-        for (int s = 0; s < g && rc == TNB_OK; ++s) {
-          const int t = w - s;
-          if (t >= 0 && t < steps) rc = spec_phase1<T, Arena>(runs[s], false, d, N - 1 - t, t, false);
-        }
-        for (int s = 0; s < g && rc == TNB_OK; ++s) {
-          const int t = w - s;
-          if (t >= 0 && t < steps) rc = spec_phase2<T, Arena>(runs[s], false, d, rmax, N - 1 - t, t, false);
-        }
-      }
-    } else {
-      for (int mu = N - 1, t = 0; mu >= 1 && rc == TNB_OK; --mu, ++t) {
-        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase1<T, Arena>(runs[s], false, d, mu, t, false);
-        if (order_phase) {
-          for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2<T, Arena>(runs[s], false, d, rmax, mu, t, false);
-        } else {
-          for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2a<T, Arena>(runs[s], false);
-          for (int stage = 0; stage <= CD_MAX_STAGES && rc == TNB_OK; ++stage)
-            for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2s<T, Arena>(runs[s], false, stage);
-          for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2b<T, Arena>(runs[s], false, d, rmax, mu, t, false);
-        }
-      }
+    // Enqueued step by step: all Gram kernels of a step, then the eigen stages of all tensors interleaved stage by
+    // stage, then every tensor's rank rule + projection.  The resident filter kernels are chained across the streams
+    // (cheb_filter.cuh), so this order keeps tensor A's Rayleigh-Ritz step in flight while tensor B's filter runs; it
+    // measured faster than enqueuing each tensor's whole eigen chain at once or a diagonal wavefront over the steps
+    // (profiles/r02_batch_schedule.md).
+    for (int mu = N - 1, t = 0; mu >= 1 && rc == TNB_OK; --mu, ++t) {
+      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase1<T, Arena>(runs[s], false, d, mu, t, false);
+      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2a<T, Arena>(runs[s], false);
+      for (int stage = 0; stage <= CD_MAX_STAGES && rc == TNB_OK; ++stage)
+        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2s<T, Arena>(runs[s], false, stage);
+      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2b<T, Arena>(runs[s], false, d, rmax, mu, t, false);
     }
     for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_end<T, Arena>(runs[s], d);
   }

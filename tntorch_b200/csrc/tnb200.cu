@@ -595,7 +595,7 @@ int tnb_gram_tc_f32(const float* A, int64_t rows, int64_t n, double* G, void* wo
                     void* stream) {
   TNB_TRY(require_device());
   if (!A || !G || !workspace) return fail(TNB_ERR_INVALID, "tnb_gram_tc_f32: null argument");
-  if (gram_use_pairs(rows, n)) return gram_tc2_f32(A, rows, n, G, nullptr, workspace, workspace_bytes, as_stream(stream));
+  if (gram_tc2_shape_ok(rows, n)) return gram_tc2_f32(A, rows, n, G, nullptr, workspace, workspace_bytes, as_stream(stream));
   return gram_tc_f32(A, rows, n, G, nullptr, workspace, workspace_bytes, as_stream(stream));
 }
 
