@@ -105,12 +105,7 @@ inline int chfsi_orthonormalize(int n, int b, TB** Xio, TB** Xtmp, ChfsiWork<TB>
     TNB_TRY((gemm_splitk<TB, TB, double, double, double>(pl, b, b, n, *Xio, b, false, *Xio, b, false,
                                                          reinterpret_cast<double*>(w.partial), w.S, b, 1.0, nullptr, 0,
                                                          0.0, nullptr, 0, 0.0, false, (double*)nullptr, 0, st)));
-    const size_t smem = (size_t)2 * b * (b | 1) * sizeof(double);
-    const bool fits = smem <= (size_t)180 * 1024;
-    static PerDeviceFlag attr_done;
-  TNB_CUDA(ensure_dyn_smem(attr_done, chol_orth_kernel<TB>, 180 * 1024));
-    chol_orth_kernel<TB><<<1, 1024, fits ? smem : 0, st>>>(w.S, b, w.jscratch, w.Tm, w.jinfo + 1, fits ? 1 : 0);
-    TNB_LAUNCH_CHECK();
+    TNB_TRY(chol_orth<TB>(w.S, b, w.jscratch, w.Tm, w.jinfo + 1, nullptr, st));
     TNB_TRY((gemm_direct<TB, TB, TB, TB>(n, b, b, *Xio, b, true, w.Tm, b, false, *Xtmp, b, (TB)1, nullptr, 0, (TB)0,
                                          nullptr, 0, (TB)0, st)));
     TB* t = *Xio; *Xio = *Xtmp; *Xtmp = t;

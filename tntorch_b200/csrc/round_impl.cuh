@@ -60,17 +60,36 @@ inline int make_round_dims(int ndim, const int64_t* shape, const int32_t* ranks_
   return TNB_OK;
 }
 
+// Work buffers of both sweeps: `cur` / `nxt` hold the core being orthogonalised (R absorbed) and the next one; Q[k] is
+// core k orthogonalised (phase A output), r_a[k] x I_k x r_a[k+1].
+template <typename T, class ArenaT>
+inline void round_carve(ArenaT& ar, const RoundDims& d, T** cur, T** nxt, std::vector<T*>& Q) {
+  size_t maxcore = 0;
+  for (int k = 0; k < d.N; ++k) maxcore = std::max<size_t>(maxcore, (size_t)d.ra[k] * d.shape[k] * d.rin[k + 1]);
+  *cur = ar.template take<T>(maxcore);
+  *nxt = ar.template take<T>(maxcore);
+  Q.assign(d.N, nullptr);
+  for (int k = 0; k < d.N; ++k) Q[k] = ar.template take<T>((size_t)d.ra[k] * d.shape[k] * std::max<int64_t>(d.ra[k + 1], 1));
+}
+
+// The two products that follow the orthogonalisation of A = core k (rowsA x cols) into fac (cols x q) and
+// Rf (q x cols, A = (A fac) Rf): Q_k = A fac (rowsA x q), and next = Rf core_{k+1} (q x ncols) carries R on.
+template <typename T>
+inline int orth_products(const T* A, int64_t rowsA, int64_t cols, const T* fac, const T* Rf, int64_t q, const T* core_next,
+                         int64_t ncols, T* Qk, T* next, cudaStream_t st) {
+  TNB_TRY((gemm_direct<T, T, T, T>(rowsA, q, cols, A, cols, true, fac, q, false, Qk, q, (T)1, nullptr, 0, (T)0, nullptr, 0,
+                                   (T)0, st)));
+  return gemm_direct<T, T, T, T>(q, ncols, cols, Rf, cols, true, core_next, ncols, false, next, ncols, (T)1, nullptr, 0, (T)0,
+                                 nullptr, 0, (T)0, st);
+}
+
 // Phase A + phase B of Tensor.round_tt (tensor.py:2008-2083) on device-resident cores.
 template <typename T, class ArenaT>
 inline int tt_round_impl(ArenaT& ar, bool dry, const T* const* cores_in, const RoundDims& d, const int32_t* rmax,
                          double eps, uint32_t flags, T* cores_out, int32_t* ranks_host, cudaStream_t st) {
   const int N = d.N;
-  StepCtx cx;
-  cx.flags = flags;
-  cx.allow_tc = false;  // TT cores are small: the generic fp64-accumulating kernels are used throughout
-  cx.st = st;
-  cx.eps_scaled2 = eps_budget2(eps, N);
-  cx.sc = ar.template take<SweepScalars>(1);
+  // TT cores are small: the generic fp64-accumulating kernels are used throughout
+  StepCtx cx(ar, N, eps, flags, false, nullptr, st, false);
   if (!dry) {
     cx.h_sc = static_cast<int*>(pinned_scratch(sizeof(SweepScalars)));
     if (!cx.h_sc) return fail(TNB_ERR_CUDA, "pinned scratch allocation failed");
@@ -84,13 +103,9 @@ inline int tt_round_impl(ArenaT& ar, bool dry, const T* const* cores_in, const R
     }
     return TNB_OK;
   }
-  // work buffers: W[k] holds the current version of core k (orthogonalised, later absorbed)
-  size_t maxcore = 0;
-  for (int k = 0; k < N; ++k) maxcore = std::max<size_t>(maxcore, (size_t)d.ra[k] * d.shape[k] * d.rin[k + 1]);
-  T* cur = ar.template take<T>(maxcore);   // R-absorbed core being orthogonalised
-  T* nxt = ar.template take<T>(maxcore);
-  std::vector<T*> Q(N, nullptr);           // orthogonalised cores (phase A output), each r_a[k]*I*r_a[k+1]
-  for (int k = 0; k < N; ++k) Q[k] = ar.template take<T>((size_t)d.ra[k] * d.shape[k] * std::max<int64_t>(d.ra[k + 1], 1));
+  T *cur, *nxt;
+  std::vector<T*> Q;
+  round_carve<T>(ar, d, &cur, &nxt, Q);
   std::vector<int64_t> r(N + 1, 1);        // actual ranks after phase A
   size_t peak = ar.off;
 
@@ -125,50 +140,29 @@ inline int tt_round_impl(ArenaT& ar, bool dry, const T* const* cores_in, const R
       bool chol_ok = false;
       if (rowsA >= cols) {
         TNB_CUDA(cudaMemsetAsync(jinfo, 0, 4 * sizeof(int), st));
-        const size_t csm = (size_t)2 * cols * (cols | 1) * sizeof(double);
-        const bool fits = csm <= (size_t)180 * 1024;
-        static PerDeviceFlag attr_done;
-  TNB_CUDA(ensure_dyn_smem(attr_done, chol_orth_kernel<T>, 180 * 1024));
-        chol_orth_kernel<T><<<1, 1024, fits ? csm : 0, st>>>(G, (int)cols, js, fac, jinfo + 1, fits ? 1 : 0, Rf);
-        TNB_LAUNCH_CHECK();
+        TNB_TRY(chol_orth<T>(G, (int)cols, js, fac, jinfo + 1, Rf, st));
         TNB_CUDA(cudaMemcpyAsync(cx.h_sc, jinfo, 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
         TNB_CUDA(cudaStreamSynchronize(st));
         chol_ok = (cx.h_sc[1] == 0);
       }
-      if (chol_ok) {
-        const int64_t q = cols;
-        r[k + 1] = q;
-        TNB_TRY((gemm_direct<T, T, T, T>(rowsA, q, cols, cur, cols, true, fac, q, false, Q[k], q, (T)1, nullptr, 0, (T)0,
-                                         nullptr, 0, (T)0, st)));
-        const int64_t ncols = d.shape[k + 1] * d.rin[k + 2];
-        TNB_TRY((gemm_direct<T, T, T, T>(q, ncols, cols, Rf, cols, true, cores_in[k + 1], ncols, false, nxt, ncols, (T)1,
-                                         nullptr, 0, (T)0, nullptr, 0, (T)0, st)));
-        T* t = cur; cur = nxt; nxt = t;
-        if (ar.off > peak) peak = ar.off;
-        ar.off = mark;
-        continue;
+      int64_t q = cols;
+      if (!chol_ok) {
+        TNB_TRY(jacobi2_eigh(G, (int)cols, (int)cols, w, V, js, jinfo, st));
+        const int64_t cap = std::min<int64_t>(rowsA, cols);
+        rank_thresh_kernel<<<1, 32, 0, st>>>(w, (int)cols, 64.0 * 2.220446049250313e-16, (int)cap, cx.sc);
+        TNB_LAUNCH_CHECK();
+        TNB_CUDA(cudaMemcpyAsync(cx.h_sc, cx.sc, sizeof(SweepScalars), cudaMemcpyDeviceToHost, st));
+        TNB_CUDA(cudaStreamSynchronize(st));
+        q = reinterpret_cast<const SweepScalars*>(cx.h_sc)->rank;
+        // fac = V_q lambda^-1/2 (cols x q);  Rf = lambda^1/2 V_q^T (q x cols)
+        scale_extract_kernel<T><<<grid_for(cols * q), 256, 0, st>>>(V, (int)cols, (int)cols, (int)q, w, fac, 1, 0);
+        TNB_LAUNCH_CHECK();
+        scale_extract_kernel<T><<<grid_for(cols * q), 256, 0, st>>>(V, (int)cols, (int)cols, (int)q, w, Rf, 2, 1);
+        TNB_LAUNCH_CHECK();
       }
-      TNB_TRY(jacobi2_eigh(G, (int)cols, (int)cols, w, V, js, jinfo, st));
-      const int64_t cap = std::min<int64_t>(rowsA, cols);
-      rank_thresh_kernel<<<1, 32, 0, st>>>(w, (int)cols, 64.0 * 2.220446049250313e-16, (int)cap, cx.sc);
-      TNB_LAUNCH_CHECK();
-      TNB_CUDA(cudaMemcpyAsync(cx.h_sc, cx.sc, sizeof(SweepScalars), cudaMemcpyDeviceToHost, st));
-      TNB_CUDA(cudaStreamSynchronize(st));
-      const SweepScalars* hs = reinterpret_cast<const SweepScalars*>(cx.h_sc);
-      const int64_t q = hs->rank;
       r[k + 1] = q;
-      // Q_k = A (V_q lambda^-1/2)   (rowsA x q)
-      scale_extract_kernel<T><<<grid_for(cols * q), 256, 0, st>>>(V, (int)cols, (int)cols, (int)q, w, fac, 1, 0);
-      TNB_LAUNCH_CHECK();
-      TNB_TRY((gemm_direct<T, T, T, T>(rowsA, q, cols, cur, cols, true, fac, q, false, Q[k], q, (T)1, nullptr, 0, (T)0,
-                                       nullptr, 0, (T)0, st)));
-      // R' = lambda^1/2 V_q^T (q x cols);  next <- R' * unfold(core_{k+1})  (q x I r'')
-      scale_extract_kernel<T><<<grid_for(cols * q), 256, 0, st>>>(V, (int)cols, (int)cols, (int)q, w, Rf, 2, 1);
-      TNB_LAUNCH_CHECK();
-      const int64_t ncols = d.shape[k + 1] * d.rin[k + 2];
-      TNB_TRY((gemm_direct<T, T, T, T>(q, ncols, cols, Rf, cols, true, cores_in[k + 1], ncols, false, nxt, ncols, (T)1,
-                                       nullptr, 0, (T)0, nullptr, 0, (T)0, st)));
-      T* t = cur; cur = nxt; nxt = t;
+      TNB_TRY(orth_products<T>(cur, rowsA, cols, fac, Rf, q, cores_in[k + 1], d.shape[k + 1] * d.rin[k + 2], Q[k], nxt, st));
+      std::swap(cur, nxt);
     }
     if (ar.off > peak) peak = ar.off;
     ar.off = mark;
@@ -219,15 +213,22 @@ __global__ void or_flag_kernel(const int* src, int* flags, int bit) {
   if (threadIdx.x == 0 && blockIdx.x == 0 && *src) atomicOr(flags, bit);
 }
 
+// Largest input rank the speculative phase A takes: the Cholesky factors L, L^-1 then stay in shared memory.
+constexpr int64_t ROUND_SPEC_MAX_RIN = 104;
+
+// A rank cap on every bond and input ranks the speculative phase A takes: the sizing pass sizes the speculative path.
+inline bool tt_round_spec_sizable(const RoundDims& d, const int32_t* rmax) {
+  if (!caps_on_every_bond(rmax, d.N)) return false;
+  for (int k = 0; k < d.N - 1; ++k)
+    if (d.rin[k + 1] > ROUND_SPEC_MAX_RIN) return false;
+  return true;
+}
+
 template <typename T>
 inline bool tt_round_spec_eligible(const RoundDims& d, const int32_t* rmax, double eps, uint32_t flags) {
-  if ((flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
-  if (!(eps_budget2(eps, d.N) < 1e-20)) return false;
-  for (int k = 0; k < d.N - 1; ++k) {
-    if (rmax[k] <= 0) return false;
+  if (!caps_decide(rmax, d.N, eps, flags) || !tt_round_spec_sizable(d, rmax)) return false;
+  for (int k = 0; k < d.N - 1; ++k)
     if (d.ra[k + 1] != d.rin[k + 1] || d.ra[k] * d.shape[k] < d.rin[k + 1]) return false;  // Cholesky-QR keeps every column
-    if (d.rin[k + 1] > JACOBI_MAX_N || d.rin[k + 1] > 104) return false;                   // L, L^-1 in shared memory
-  }
   for (int mu = d.N - 1; mu >= 1; --mu)
     if (!spec_step_ok<T>(d.ra[mu], d.shape[mu] * d.rcap[mu + 1], d.rcap[mu], false)) return false;
   return true;
@@ -237,21 +238,11 @@ template <typename T, class ArenaT>
 inline int tt_round_spec_enqueue(ArenaT& ar, bool dry, const T* const* cores_in, const RoundDims& d, const int32_t* rmax,
                                  double eps, uint32_t flags, T* cores_out, SpecHostBack* hb, cudaStream_t st) {
   const int N = d.N;
-  StepCtx cx;
-  cx.flags = flags;
-  cx.allow_tc = false;
-  cx.st = st;
-  cx.eps_scaled2 = eps_budget2(eps, N);
-  cx.sc = ar.template take<SweepScalars>(1);
-  cx.d_flags = ar.template take<int>(4);
-  cx.d_ranks = ar.template take<int32_t>(N + 1);
+  StepCtx cx(ar, N, eps, flags, false, nullptr, st, true);
   int* d_chol = ar.template take<int>(4);
-  size_t maxcore = 0;
-  for (int k = 0; k < N; ++k) maxcore = std::max<size_t>(maxcore, (size_t)d.ra[k] * d.shape[k] * d.rin[k + 1]);
-  T* cur = ar.template take<T>(maxcore);
-  T* nxt = ar.template take<T>(maxcore);
-  std::vector<T*> Q(N, nullptr);
-  for (int k = 0; k < N; ++k) Q[k] = ar.template take<T>((size_t)d.ra[k] * d.shape[k] * std::max<int64_t>(d.ra[k + 1], 1));
+  T *cur, *nxt;
+  std::vector<T*> Q;
+  round_carve<T>(ar, d, &cur, &nxt, Q);
   size_t peak = ar.off;
   if (!dry) {
     TNB_CUDA(cudaMemsetAsync(cx.d_flags, 0, 4 * sizeof(int), st));
@@ -275,17 +266,9 @@ inline int tt_round_spec_enqueue(ArenaT& ar, bool dry, const T* const* cores_in,
       TNB_TRY((gemm_splitk<T, T, double, double, float>(pl, cols, cols, rowsA, cur, cols, false, cur, cols, false, partial, G,
                                                         cols, 1.0, nullptr, 0, 0.0, nullptr, 0, 0.0, true, (float*)nullptr, 0,
                                                         st)));
-      const size_t csm = (size_t)2 * cols * (cols | 1) * sizeof(double);
-      static PerDeviceFlag attr_done;
-      TNB_CUDA(ensure_dyn_smem(attr_done, chol_orth_kernel<T>, 180 * 1024));
-      chol_orth_kernel<T><<<1, 1024, csm, st>>>(G, (int)cols, js, fac, d_chol, 1, Rf);
-      TNB_LAUNCH_CHECK();
-      TNB_TRY((gemm_direct<T, T, T, T>(rowsA, cols, cols, cur, cols, true, fac, cols, false, Q[k], cols, (T)1, nullptr, 0,
-                                       (T)0, nullptr, 0, (T)0, st)));
-      const int64_t ncols = d.shape[k + 1] * d.rin[k + 2];
-      TNB_TRY((gemm_direct<T, T, T, T>(cols, ncols, cols, Rf, cols, true, cores_in[k + 1], ncols, false, nxt, ncols, (T)1,
-                                       nullptr, 0, (T)0, nullptr, 0, (T)0, st)));
-      T* t = cur; cur = nxt; nxt = t;
+      TNB_TRY(chol_orth<T>(G, (int)cols, js, fac, d_chol, Rf, st));  // L, L^-1 in shared memory: cols <= ROUND_SPEC_MAX_RIN
+      TNB_TRY(orth_products<T>(cur, rowsA, cols, fac, Rf, cols, cores_in[k + 1], d.shape[k + 1] * d.rin[k + 2], Q[k], nxt, st));
+      std::swap(cur, nxt);
     }
     ar.off = mark;
   }
@@ -327,46 +310,26 @@ inline int tt_round_spec_enqueue(ArenaT& ar, bool dry, const T* const* cores_in,
   return TNB_OK;
 }
 
-inline void tt_round_spec_ranks(const RoundDims& d, int32_t* ranks_host) {
-  ranks_host[0] = 1;
-  ranks_host[d.N] = 1;
-  for (int mu = 1; mu < d.N; ++mu) ranks_host[mu] = (int32_t)d.rcap[mu];
-}
-
-// Dispatcher: speculative rounding when eligible, host-driven rounding otherwise and as the fallback.
+// The speculative rounding never returns TNB_ERR_NOCONV: its steps are eligible only for the direct eigensolver
+// (allow_tc is false), whose solve is enqueued and cannot report non-convergence.
 template <typename T, class ArenaT>
 inline int tt_round_any(ArenaT& ar, bool dry, const T* const* cores_in, const RoundDims& d, const int32_t* rmax, double eps,
-                        uint32_t flags, T* cores_out, int32_t* ranks_host, cudaStream_t st, int* speculative_out = nullptr) {
-  const size_t base = ar.off;
-  if (speculative_out) *speculative_out = 0;
-  if (dry) {
-    size_t need = 0;
-    bool caps = rmax != nullptr && d.N >= 2;
-    for (int k = 0; caps && k < d.N - 1; ++k) caps = rmax[k] > 0 && d.rin[k + 1] <= 104;
-    if (caps) {
-      const int rc = tt_round_spec_enqueue<T>(ar, true, cores_in, d, rmax, eps, flags, cores_out, nullptr, st);
-      if (rc == TNB_OK) need = ar.off - base;
-      ar.off = base;
-    }
-    const int rc = tt_round_impl<T>(ar, true, cores_in, d, rmax, eps, flags, cores_out, ranks_host, st);
-    if (rc == TNB_OK && need > ar.off - base) ar.off = base + need;
-    return rc;
-  }
-  if (tt_round_spec_eligible<T>(d, rmax, eps, flags)) {
-    SpecHostBack* hb = static_cast<SpecHostBack*>(pinned_scratch(sizeof(SpecHostBack)));
-    if (!hb) return fail(TNB_ERR_CUDA, "pinned scratch allocation failed");
-    const int rc = tt_round_spec_enqueue<T>(ar, false, cores_in, d, rmax, eps, flags, cores_out, hb, st);
-    TNB_CUDA(cudaStreamSynchronize(st));
-    if (rc == TNB_OK && hb->flags[0] == 0) {
-      tt_round_spec_ranks(d, ranks_host);
-      if (speculative_out) *speculative_out = 1;
-      return TNB_OK;
-    }
-    if (rc != TNB_OK && rc != TNB_ERR_UNSUPPORTED) return rc;
-    ar.off = base;
-    ar.ok = true;
-  }
-  return tt_round_impl<T>(ar, false, cores_in, d, rmax, eps, flags, cores_out, ranks_host, st);
+                        uint32_t flags, T* cores_out, int32_t* ranks_host, cudaStream_t st, SweepInfo* info = nullptr) {
+  const bool try_spec = dry ? tt_round_spec_sizable(d, rmax) : tt_round_spec_eligible<T>(d, rmax, eps, flags);
+  return speculate_or_fall_back(
+      ar, dry, try_spec, info,
+      [&](bool dr, int* spec_flags) {
+        if (dr) return tt_round_spec_enqueue<T>(ar, true, cores_in, d, rmax, eps, flags, cores_out, nullptr, st);
+        SpecHostBack* hb = static_cast<SpecHostBack*>(pinned_scratch(sizeof(SpecHostBack)));
+        if (!hb) return fail(TNB_ERR_CUDA, "pinned scratch allocation failed");
+        const int rc = tt_round_spec_enqueue<T>(ar, false, cores_in, d, rmax, eps, flags, cores_out, hb, st);
+        TNB_CUDA(cudaStreamSynchronize(st));
+        if (rc != TNB_OK) return rc;
+        *spec_flags = hb->flags[0];
+        if (*spec_flags == 0) ranks_from_caps(d.rcap, ranks_host);
+        return TNB_OK;
+      },
+      [&](bool dr, int) { return tt_round_impl<T>(ar, dr, cores_in, d, rmax, eps, flags, cores_out, ranks_host, st); });
 }
 
 // A batch of TT tensors with one rank profile: every tensor's two sweeps on its own internal stream, one synchronisation.
@@ -376,52 +339,26 @@ inline int tt_round_batch_impl(void* workspace, size_t per_tensor_bytes, int inf
                                T* const* cores_out, int32_t* ranks_host, int32_t* spec_host, cudaStream_t st) {
   const int N = d.N;
   char* ws = static_cast<char*>(workspace);
-  const bool spec = batch > 1 && inflight > 1 && tt_round_spec_eligible<T>(d, rmax, eps, flags);
-  if (!spec) {
-    for (int i = 0; i < batch; ++i) {
-      Arena ar(ws, per_tensor_bytes);
-      int sp = 0;
-      TNB_TRY((tt_round_any<T, Arena>(ar, false, cores_in + (size_t)i * N, d, rmax, eps, flags, cores_out[i],
-                                      ranks_host + (size_t)i * (N + 1), st, &sp)));
-      if (spec_host) spec_host[i] = sp;
+  auto in = [&](int i) { return cores_in + (size_t)i * N; };
+  auto ranks = [&](int i) { return ranks_host + (size_t)i * (N + 1); };
+  auto one = [&](Arena& ar, int i, SweepInfo* info) {
+    return tt_round_any<T, Arena>(ar, false, in(i), d, rmax, eps, flags, cores_out[i], ranks(i), st, info);
+  };
+  auto enqueue = [&](cudaStream_t* streams, int inflight, SpecHostBack* hbs) {
+    int rc = TNB_OK;
+    for (int i = 0; i < batch && rc == TNB_OK; ++i) {
+      const int s = i % inflight;  // tensor i + inflight reuses workspace slice s on the same stream: ordered
+      Arena ar(ws + (size_t)s * per_tensor_bytes, per_tensor_bytes);
+      rc = tt_round_spec_enqueue<T>(ar, false, in(i), d, rmax, eps, flags, cores_out[i], hbs + i, streams[s]);
     }
-    return TNB_OK;
-  }
-  if (inflight > TNB_BATCH_MAX_INFLIGHT) inflight = TNB_BATCH_MAX_INFLIGHT;
-  if (inflight > batch) inflight = batch;
-  StreamPool& pool = StreamPool::get();
-  std::lock_guard<std::mutex> lk(pool.mu);
-  TNB_TRY(pool.ensure());
-  SpecHostBack* hbs = static_cast<SpecHostBack*>(pinned_scratch((size_t)batch * sizeof(SpecHostBack)));
-  if (!hbs) return fail(TNB_ERR_CUDA, "pinned scratch allocation failed");
-  TNB_CUDA(cudaEventRecord(pool.ev[TNB_BATCH_MAX_INFLIGHT], st));
-  for (int s = 0; s < inflight; ++s) TNB_CUDA(cudaStreamWaitEvent(pool.st[s], pool.ev[TNB_BATCH_MAX_INFLIGHT], 0));
-  int rc = TNB_OK;
-  for (int i = 0; i < batch && rc == TNB_OK; ++i) {
-    const int s = i % inflight;  // tensor i + inflight reuses workspace slice s on the same stream: ordered
-    Arena ar(ws + (size_t)s * per_tensor_bytes, per_tensor_bytes);
-    rc = tt_round_spec_enqueue<T>(ar, false, cores_in + (size_t)i * N, d, rmax, eps, flags, cores_out[i], hbs + i, pool.st[s]);
-  }
-  for (int s = 0; s < inflight; ++s) {
-    cudaEventRecord(pool.ev[s], pool.st[s]);
-    cudaStreamWaitEvent(st, pool.ev[s], 0);
-  }
-  TNB_CUDA(cudaStreamSynchronize(st));
-  if (rc != TNB_OK && rc != TNB_ERR_UNSUPPORTED) return rc;
-  std::vector<int> bad(batch, 0);
-  for (int i = 0; i < batch; ++i) bad[i] = (rc != TNB_OK) || hbs[i].flags[0] != 0;
-  for (int i = 0; i < batch; ++i) {
-    int32_t* rk = ranks_host + (size_t)i * (N + 1);
-    if (!bad[i]) {
-      tt_round_spec_ranks(d, rk);
-      if (spec_host) spec_host[i] = 1;
-      continue;
-    }
-    Arena ar(ws, per_tensor_bytes);
-    TNB_TRY((tt_round_impl<T, Arena>(ar, false, cores_in + (size_t)i * N, d, rmax, eps, flags, cores_out[i], rk, st)));
-    if (spec_host) spec_host[i] = 0;
-  }
-  return TNB_OK;
+    return rc;
+  };
+  auto accept = [&](int i, const SpecHostBack&) { ranks_from_caps(d.rcap, ranks(i)); };
+  auto repeat = [&](Arena& ar, int i, int) {
+    return tt_round_impl<T, Arena>(ar, false, in(i), d, rmax, eps, flags, cores_out[i], ranks(i), st);
+  };
+  const bool spec = tt_round_spec_eligible<T>(d, rmax, eps, flags);
+  return spec_batch(workspace, per_tensor_bytes, inflight, batch, spec, spec_host, st, one, enqueue, accept, repeat);
 }
 
 // ---------------------------------------------------------------------------------------------

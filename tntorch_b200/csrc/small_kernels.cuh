@@ -295,6 +295,18 @@ __global__ void __launch_bounds__(1024) chol_orth_kernel(const double* __restric
   chol_orth_device<TB>(S, b, scratch, T, flag, use_smem, Rout, chol_smem_dyn);
 }
 
+// chol_orth_kernel on `st`: L and L^-1 in shared memory when they fit its 180 KB, in `scratch` otherwise.
+template <typename TB>
+inline int chol_orth(const double* S, int b, double* scratch, TB* T, int* flag, TB* Rout, cudaStream_t st) {
+  const size_t smem = (size_t)2 * b * (b | 1) * sizeof(double);
+  const bool fits = smem <= (size_t)180 * 1024;
+  static PerDeviceFlag attr_done;
+  TNB_CUDA(ensure_dyn_smem(attr_done, chol_orth_kernel<TB>, 180 * 1024));
+  chol_orth_kernel<TB><<<1, 1024, fits ? smem : 0, st>>>(S, b, scratch, T, flag, fits ? 1 : 0, Rout);
+  TNB_LAUNCH_CHECK();
+  return TNB_OK;
+}
+
 inline int grid_for(int64_t n, int block = 256, int cap = 4096) {
   int64_t g = ceil_div<int64_t>(n, block);
   if (g < 1) g = 1;

@@ -339,7 +339,19 @@ struct StepCtx {
   bool exact_gram = false;      // a TF32 Gram was rejected for this tensor: take the exact-product Gram throughout
   // speculative (sync-free) sweep
   int* d_flags = nullptr;       // device flags raised by spec_check_kernel / cd_finish_kernel
-  int32_t* d_ranks = nullptr;   // device copy of the ranks the rule chose, [N + 1]
+  int32_t* d_ranks = nullptr;   // the ranks the rule chose, [N + 1] (written by spec_check_kernel, not read back)
+
+  StepCtx() = default;
+  // Carves the device scalars of an N-mode sweep, and for a speculative one its device flags and ranks.
+  template <class ArenaT>
+  StepCtx(ArenaT& ar, int N, double eps, uint32_t flags_, bool allow_tc_, SweepInfo* info_, cudaStream_t st_, bool speculative)
+      : flags(flags_), allow_tc(allow_tc_), eps_scaled2(eps_budget2(eps, N)), info(info_), st(st_) {
+    sc = ar.template take<SweepScalars>(1);
+    if (speculative) {
+      d_flags = ar.template take<int>(4);
+      d_ranks = ar.template take<int32_t>(N + 1);
+    }
+  }
 };
 
 // The two factors of a truncation step from the leading eigenpairs (w, V) of the Gram matrix on the smaller side of C:
@@ -583,14 +595,8 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
                            uint32_t flags, T* cores, int32_t* ranks_host, SweepInfo* info, cudaStream_t st,
                            bool exact_gram = false) {
   const int N = d.N;
-  StepCtx cx;
-  cx.flags = flags;
+  StepCtx cx(ar, N, eps, flags, tc_allowed(flags, dry), info, st, false);
   cx.exact_gram = exact_gram;
-  cx.allow_tc = tc_allowed(flags, dry);
-  cx.info = info;
-  cx.st = st;
-  cx.eps_scaled2 = eps_budget2(eps, N);
-  cx.sc = ar.template take<SweepScalars>(1);
   Prof& prof = Prof::get();
   prof.on = !dry && (flags & TNB_FLAG_PROFILE);
   prof.used = 0;
@@ -643,61 +649,61 @@ inline int ttsvd_sync_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
 // ---------------------------------------------------------------------------------------------
 // Speculative dense TT-SVD: the whole right-to-left sweep enqueued in one go, ONE synchronisation at the end.
 // ---------------------------------------------------------------------------------------------
-template <typename T>
-inline bool spec_eligible(const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, bool allow_tc) {
-  if ((flags & TNB_FLAG_NO_SPECULATE) || d.N < 2 || !rmax) return false;
-  if (!(eps_budget2(eps, d.N) < 1e-20)) return false;  // an active eps budget decides ranks: host-driven path
-  for (int mu = d.N - 1; mu >= 1; --mu) {
-    if (rmax[mu - 1] <= 0) return false;
-    if (!spec_step_ok<T>(d.rows[mu], d.shape[mu] * d.rcap[mu + 1], d.rcap[mu], allow_tc)) return false;
-  }
+// A rank cap on every bond of an N-mode train: the condition under which the sizing pass sizes a speculative path.
+inline bool caps_on_every_bond(const int32_t* rmax, int N) {
+  if (N < 2 || !rmax) return false;
+  for (int k = 0; k < N - 1; ++k)
+    if (rmax[k] <= 0) return false;
   return true;
 }
+// The speculative paths assume every rank is its cap: the caller did not opt out, a cap decides every bond, and no
+// active eps budget decides ranks instead.
+inline bool caps_decide(const int32_t* rmax, int N, double eps, uint32_t flags) {
+  return !(flags & TNB_FLAG_NO_SPECULATE) && eps_budget2(eps, N) < 1e-20 && caps_on_every_bond(rmax, N);
+}
 
-struct SpecOutcome {
-  int flags = 0;
-  bool ran = false;
-};
+template <typename T>
+inline bool spec_eligible(const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, bool allow_tc) {
+  if (!caps_decide(rmax, d.N, eps, flags)) return false;
+  for (int mu = d.N - 1; mu >= 1; --mu)
+    if (!spec_step_ok<T>(d.rows[mu], d.shape[mu] * d.rcap[mu + 1], d.rcap[mu], allow_tc)) return false;
+  return true;
+}
 
 struct SpecHostBack {  // pinned read-back of one speculative sweep
   SweepScalars sc;
   int flags[4];
-  int32_t ranks[64];
 };
+
+// The ranks of an accepted speculation: every bond took its cap.
+inline void ranks_from_caps(const std::vector<int64_t>& rcap, int32_t* ranks_host) {
+  const int N = (int)rcap.size() - 1;
+  ranks_host[0] = 1;
+  ranks_host[N] = 1;
+  for (int mu = 1; mu < N; ++mu) ranks_host[mu] = (int32_t)rcap[mu];
+}
 
 // One tensor of a speculative sweep (or of a batch of them): its arena, device scalars, carries and position.
 template <typename T, class ArenaT>
 struct SpecRun {
   ArenaT* ar = nullptr;
   StepCtx cx;
-  SweepInfo info_local;
   const T* C = nullptr;
   T* carry[2] = {nullptr, nullptr};
   T* cores = nullptr;
   SpecStep<T> step;
   size_t mark = 0, peak = 0;
-  SpecHostBack* hb = nullptr;
 };
 
 template <typename T, class ArenaT>
 inline int spec_begin(SpecRun<T, ArenaT>& r, ArenaT& ar, bool dry, const T* data, const SweepDims& d, double eps,
-                      uint32_t flags, T* cores, SweepInfo* info, cudaStream_t st, SpecHostBack* hb) {
-  const int N = d.N;
+                      uint32_t flags, T* cores, SweepInfo* info, cudaStream_t st) {
   r.ar = &ar;
-  r.cx = StepCtx();
-  r.cx.flags = flags;
-  r.cx.allow_tc = tc_allowed(flags, dry);
-  r.cx.info = info;
-  r.cx.st = st;
-  r.cx.eps_scaled2 = eps_budget2(eps, N);
-  r.cx.sc = ar.template take<SweepScalars>(1);
-  r.cx.d_flags = ar.template take<int>(4);
-  r.cx.d_ranks = ar.template take<int32_t>(N + 1);
+  r.cx = StepCtx(ar, d.N, eps, flags, tc_allowed(flags, dry), info, st, true);
   carry_carve<T>(ar, d, r.carry);
   r.C = data;
   r.cores = cores;
   r.peak = ar.off;
-  r.hb = hb;
   if (!dry) TNB_CUDA(cudaMemsetAsync(r.cx.d_flags, 0, 4 * sizeof(int), st));
   return TNB_OK;
 }
@@ -741,37 +747,31 @@ inline int spec_phase2(SpecRun<T, ArenaT>& r, bool dry, const SweepDims& d, cons
   return spec_phase2b<T, ArenaT>(r, dry, d, rmax, mu, t, prof_on);
 }
 template <typename T, class ArenaT>
-inline int spec_end(SpecRun<T, ArenaT>& r, const SweepDims& d) {
+inline int spec_end(SpecRun<T, ArenaT>& r, const SweepDims& d, SpecHostBack* hb) {
   cudaStream_t st = r.cx.st;
-  const int N = d.N;
   TNB_CUDA(cudaMemcpyAsync(r.cores + d.slot[0], r.C, sizeof(T) * (size_t)d.shape[0] * (size_t)d.rcap[1],
                            cudaMemcpyDeviceToDevice, st));
-  TNB_CUDA(cudaMemcpyAsync(&r.hb->sc, r.cx.sc, sizeof(SweepScalars), cudaMemcpyDeviceToHost, st));
-  TNB_CUDA(cudaMemcpyAsync(r.hb->flags, r.cx.d_flags, 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
-  TNB_CUDA(cudaMemcpyAsync(r.hb->ranks, r.cx.d_ranks, (size_t)(N + 1) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  TNB_CUDA(cudaMemcpyAsync(&hb->sc, r.cx.sc, sizeof(SweepScalars), cudaMemcpyDeviceToHost, st));
+  TNB_CUDA(cudaMemcpyAsync(hb->flags, r.cx.d_flags, 4 * sizeof(int), cudaMemcpyDeviceToHost, st));
   return TNB_OK;
 }
-// after the stream has been synchronised
-inline void spec_collect(const SpecHostBack* hb, const SweepDims& d, int32_t* ranks_host, SweepInfo* info, SpecOutcome* out) {
-  const int N = d.N;
-  out->ran = true;
-  out->flags = hb->flags[0];
-  ranks_host[0] = 1;
-  ranks_host[N] = 1;
-  for (int mu = 1; mu < N; ++mu) ranks_host[mu] = (int32_t)d.rcap[mu];  // the flags say whether the rule agreed
+// An accepted sweep, after the stream has been synchronised: ranks = caps, the scalars from the read-back.
+inline void spec_accept(const SpecHostBack& hb, const SweepDims& d, int32_t* ranks_host, SweepInfo* info) {
+  ranks_from_caps(d.rcap, ranks_host);
   if (info) {
-    info->norm = std::sqrt(hb->sc.norm2 > 0 ? hb->sc.norm2 : 0.0);
-    info->chfsi_products += hb->flags[1];
-    info->rr_solves += hb->flags[2];
-    info->rr_sweeps += hb->flags[3];
-    info->fused_filters += hb->flags[2] - info->eig_solves;  // every Rayleigh-Ritz step but the first of a solve follows a filter
+    info->norm = std::sqrt(hb.sc.norm2 > 0 ? hb.sc.norm2 : 0.0);
+    info->chfsi_products += hb.flags[1];
+    info->rr_solves += hb.flags[2];
+    info->rr_sweeps += hb.flags[3];
+    info->fused_filters += hb.flags[2] - info->eig_solves;  // every Rayleigh-Ritz step but the first of a solve follows a filter
   }
 }
 
+// A real run enqueues the sweep, synchronises once and returns the device flags; the result stands when they are 0.
 template <typename T, class ArenaT>
 inline int ttsvd_spec_impl(ArenaT& ar, bool dry, const T* data, const SweepDims& d, const int32_t* rmax, double eps,
                            uint32_t flags, T* cores, int32_t* ranks_host, SweepInfo* info, cudaStream_t st,
-                           SpecOutcome* out) {
+                           int* spec_flags) {
   const int N = d.N;
   Prof& prof = Prof::get();
   prof.on = !dry && (flags & TNB_FLAG_PROFILE);
@@ -783,7 +783,7 @@ inline int ttsvd_spec_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
     if (!hb) return fail(TNB_ERR_CUDA, "pinned scratch allocation failed");
   }
   SpecRun<T, ArenaT> r;
-  TNB_TRY((spec_begin<T, ArenaT>(r, ar, dry, data, d, eps, flags, cores, info, st, hb)));
+  TNB_TRY((spec_begin<T, ArenaT>(r, ar, dry, data, d, eps, flags, cores, info, st)));
   for (int mu = N - 1, t = 0; mu >= 1; --mu, ++t) {
     int rc = spec_phase1<T, ArenaT>(r, dry, d, mu, t, prof_on);
     if (rc == TNB_OK) rc = spec_phase2<T, ArenaT>(r, dry, d, rmax, mu, t, prof_on);
@@ -797,53 +797,70 @@ inline int ttsvd_spec_impl(ArenaT& ar, bool dry, const T* data, const SweepDims&
     ar.off = r.peak;
     return TNB_OK;
   }
-  TNB_TRY((spec_end<T, ArenaT>(r, d)));
+  TNB_TRY((spec_end<T, ArenaT>(r, d, hb)));
   TNB_CUDA(cudaStreamSynchronize(st));
-  spec_collect(hb, d, ranks_host, info, out);
+  *spec_flags = hb->flags[0];
+  if (*spec_flags == 0) spec_accept(*hb, d, ranks_host, info);
   if (prof_on && info) prof.report(info);
   prof.on = false;
   return TNB_OK;
 }
 
-// Dispatcher: speculative sweep when a rank cap decides every bond, host-driven sweep otherwise and as the fallback.
+// ---------------------------------------------------------------------------------------------
+// Speculate, then fall back: the policy of dense TT-SVD (ttsvd_impl) and TT rounding (tt_round_any).
+//   spec(dry, &flags): a real run enqueues the speculative path, synchronises once, returns the device flags and, when
+//                      they are 0, writes the result
+//   sync(dry, flags):  the host-driven path, given the flags of the rejected speculation (0 when none ran)
+// The sizing pass cannot ask the device what it supports: there `try_spec` is the caller's precondition instead of its
+// eligibility test, and the workspace fits the larger path.  A flag, TNB_ERR_UNSUPPORTED or TNB_ERR_NOCONV restores
+// the caller's info and arena and runs the host-driven path; any other error is returned.
+// ---------------------------------------------------------------------------------------------
+template <class ArenaT, class Spec, class Sync>
+inline int speculate_or_fall_back(ArenaT& ar, bool dry, bool try_spec, SweepInfo* info, Spec spec, Sync sync) {
+  const size_t base = ar.off;
+  if (dry) {
+    size_t need_spec = 0;
+    if (try_spec) {
+      int flags = 0;
+      if (spec(true, &flags) == TNB_OK) need_spec = ar.off - base;
+      ar.off = base;
+    }
+    const int rc = sync(true, 0);
+    if (rc == TNB_OK && need_spec > ar.off - base) ar.off = base + need_spec;
+    return rc;
+  }
+  if (!try_spec) return sync(false, 0);
+  SweepInfo saved;
+  if (info) saved = *info;
+  int flags = 0;
+  const int rc = spec(false, &flags);
+  if (rc == TNB_OK && flags == 0) {
+    if (info) info->speculative = 1;
+    return TNB_OK;
+  }
+  if (rc != TNB_OK && rc != TNB_ERR_UNSUPPORTED && rc != TNB_ERR_NOCONV) return rc;
+  if (info) {
+    *info = saved;
+    info->spec_flags = flags;
+  }
+  ar.off = base;
+  ar.ok = true;
+  return sync(false, flags);
+}
+
 template <typename T, class ArenaT>
 inline int ttsvd_impl(ArenaT& ar, bool dry, const T* data, const SweepDims& d, const int32_t* rmax, double eps,
                       uint32_t flags, T* cores, int32_t* ranks_host, SweepInfo* info, cudaStream_t st) {
-  // the sizing pass cannot ask the device what it supports: size for both paths
-  const bool spec = dry ? (d.N >= 2 && rmax != nullptr) : spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
-  const size_t base = ar.off;
-  size_t need_spec = 0;
-  if (spec) {
-    if (dry) {
-      bool all_caps = true;
-      for (int mu = 1; mu < d.N; ++mu) all_caps = all_caps && rmax[mu - 1] > 0;
-      if (all_caps) {
-        SpecOutcome o;
-        const int rc = ttsvd_spec_impl<T>(ar, true, data, d, rmax, eps, flags, cores, ranks_host, info, st, &o);
-        if (rc == TNB_OK) need_spec = ar.off - base;
-        ar.off = base;
-      }
-    } else {
-      SpecOutcome o;
-      SweepInfo saved;
-      if (info) saved = *info;
-      const int rc = ttsvd_spec_impl<T>(ar, false, data, d, rmax, eps, flags, cores, ranks_host, info, st, &o);
-      if (rc == TNB_OK && o.ran && o.flags == 0) {
-        if (info) info->speculative = 1;
-        return TNB_OK;
-      }
-      if (rc != TNB_OK && rc != TNB_ERR_UNSUPPORTED && rc != TNB_ERR_NOCONV) return rc;
-      // the device disagreed with the speculation (or could not run the sync-free solver): host-driven sweep;
-      // bit 0 = the TF32 Gram is too coarse for this spectrum, so the repeat takes exact-product Gram matrices
-      if (info) { *info = saved; info->spec_flags = o.flags; }
-      ar.off = base;
-      ar.ok = true;
-      return ttsvd_sync_impl<T>(ar, false, data, d, rmax, eps, flags, cores, ranks_host, info, st, (o.flags & 1) != 0);
-    }
-  }
-  const int rc = ttsvd_sync_impl<T>(ar, dry, data, d, rmax, eps, flags, cores, ranks_host, info, st);
-  if (dry && rc == TNB_OK && need_spec > ar.off - base) ar.off = base + need_spec;
-  return rc;
+  const bool try_spec = dry ? caps_on_every_bond(rmax, d.N) : spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
+  return speculate_or_fall_back(
+      ar, dry, try_spec, info,
+      [&](bool dr, int* spec_flags) {
+        return ttsvd_spec_impl<T>(ar, dr, data, d, rmax, eps, flags, cores, ranks_host, info, st, spec_flags);
+      },
+      // flag bit 0: the TF32 Gram is too coarse for this spectrum, so the repeat takes exact-product Gram matrices
+      [&](bool dr, int spec_flags) {
+        return ttsvd_sync_impl<T>(ar, dr, data, d, rmax, eps, flags, cores, ranks_host, info, st, (spec_flags & 1) != 0);
+      });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -872,19 +889,19 @@ struct StreamPool {
   }
 };
 
-template <typename T>
-inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflight, const T* const* data, int batch,
-                            const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, T* const* cores,
-                            int32_t* ranks_host, double* norms_host, int32_t* spec_host, cudaStream_t st) {
-  const int N = d.N;
-  const bool spec = batch > 0 && spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
-  char* ws = static_cast<char*>(workspace);
-  if (!spec || inflight < 2 || batch < 2) {  // one at a time through the dispatcher (speculative when eligible)
+// The batch form of speculate_or_fall_back over workspace slices of `per_tensor_bytes`.  Without speculation, or with
+// fewer than two tensors or slices, tensor i goes through one(ar, i, info).  Otherwise enqueue(streams, n, hbs) puts the
+// speculative work of every tensor on n internal streams forked from `st` (tensor i reads back into hbs[i]), the streams
+// are joined back and the host synchronises once; then tensor i is accepted, accept(i, hbs[i]), or repeated host-driven
+// on `st`, repeat(ar, i, flags).  spec_host[i] (may be null) says which.
+template <class One, class Enqueue, class Accept, class Repeat>
+inline int spec_batch(void* workspace, size_t per_tensor_bytes, int inflight, int batch, bool spec, int32_t* spec_host,
+                      cudaStream_t st, One one, Enqueue enqueue, Accept accept, Repeat repeat) {
+  if (!spec || inflight < 2 || batch < 2) {
     for (int i = 0; i < batch; ++i) {
-      Arena ar(ws, per_tensor_bytes);
+      Arena ar(workspace, per_tensor_bytes);
       SweepInfo info;
-      TNB_TRY((ttsvd_impl<T, Arena>(ar, false, data[i], d, rmax, eps, flags, cores[i], ranks_host + (size_t)i * (N + 1), &info, st)));
-      if (norms_host) norms_host[i] = info.norm;
+      TNB_TRY(one(ar, i, &info));
       if (spec_host) spec_host[i] = info.speculative;
     }
     return TNB_OK;
@@ -899,32 +916,7 @@ inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflig
   // fork: the internal streams start after whatever the caller enqueued on `st`
   TNB_CUDA(cudaEventRecord(pool.ev[TNB_BATCH_MAX_INFLIGHT], st));
   for (int s = 0; s < inflight; ++s) TNB_CUDA(cudaStreamWaitEvent(pool.st[s], pool.ev[TNB_BATCH_MAX_INFLIGHT], 0));
-  const uint32_t bflags = (flags | TNB_FLAG_CONCURRENT) & ~TNB_FLAG_PROFILE;
-  std::vector<SweepInfo> infos(batch);
-  int rc = TNB_OK;
-  for (int g0 = 0; g0 < batch && rc == TNB_OK; g0 += inflight) {
-    const int g = std::min(inflight, batch - g0);
-    std::vector<Arena> arenas;
-    arenas.reserve(g);
-    std::vector<SpecRun<T, Arena>> runs(g);
-    for (int s = 0; s < g; ++s) arenas.emplace_back(ws + (size_t)s * per_tensor_bytes, per_tensor_bytes);
-    for (int s = 0; s < g && rc == TNB_OK; ++s)
-      rc = spec_begin<T, Arena>(runs[s], arenas[s], false, data[g0 + s], d, eps, bflags, cores[g0 + s], &infos[g0 + s],
-                                pool.st[s], hbs + g0 + s);
-    // Enqueued step by step: all Gram kernels of a step, then the eigen stages of all tensors interleaved stage by
-    // stage, then every tensor's rank rule + projection.  The resident filter kernels are chained across the streams
-    // (cheb_filter.cuh), so this order keeps tensor A's Rayleigh-Ritz step in flight while tensor B's filter runs; it
-    // measured faster than enqueuing each tensor's whole eigen chain at once or a diagonal wavefront over the steps
-    // (profiles/r02_batch_schedule.md).
-    for (int mu = N - 1, t = 0; mu >= 1 && rc == TNB_OK; --mu, ++t) {
-      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase1<T, Arena>(runs[s], false, d, mu, t, false);
-      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2a<T, Arena>(runs[s], false);
-      for (int stage = 0; stage <= CD_MAX_STAGES && rc == TNB_OK; ++stage)
-        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2s<T, Arena>(runs[s], false, stage);
-      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2b<T, Arena>(runs[s], false, d, rmax, mu, t, false);
-    }
-    for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_end<T, Arena>(runs[s], d);
-  }
+  const int rc = enqueue(pool.st, inflight, hbs);
   // join: the caller's stream continues after every internal stream; then the one host synchronisation
   for (int s = 0; s < inflight; ++s) {
     cudaEventRecord(pool.ev[s], pool.st[s]);
@@ -933,25 +925,76 @@ inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflig
   TNB_CUDA(cudaStreamSynchronize(st));
   if (rc != TNB_OK && rc != TNB_ERR_UNSUPPORTED && rc != TNB_ERR_NOCONV) return rc;
   // read every outcome out of the pinned block first: the host-driven repeats below reuse that scratch
-  std::vector<SpecOutcome> outs(batch);
-  for (int i = 0; i < batch; ++i)
-    if (rc == TNB_OK) spec_collect(hbs + i, d, ranks_host + (size_t)i * (N + 1), &infos[i], &outs[i]);
+  std::vector<int> flags(batch, 0);
+  for (int i = 0; i < batch && rc == TNB_OK; ++i) {
+    flags[i] = hbs[i].flags[0];
+    if (flags[i] == 0) accept(i, hbs[i]);
+  }
   for (int i = 0; i < batch; ++i) {
-    int32_t* rk = ranks_host + (size_t)i * (N + 1);
-    if (rc == TNB_OK && outs[i].flags == 0) {
-      if (norms_host) norms_host[i] = infos[i].norm;
-      if (spec_host) spec_host[i] = 1;
-      continue;
+    const bool accepted = rc == TNB_OK && flags[i] == 0;
+    if (!accepted) {
+      Arena ar(workspace, per_tensor_bytes);
+      TNB_TRY(repeat(ar, i, flags[i]));
     }
-    // repeat this tensor on the host-driven path (exact Gram when the TF32 one was rejected)
-    Arena ar(ws, per_tensor_bytes);
-    SweepInfo info;
-    TNB_TRY((ttsvd_sync_impl<T, Arena>(ar, false, data[i], d, rmax, eps, flags & ~TNB_FLAG_PROFILE, cores[i], rk, &info, st,
-                                       (outs[i].flags & 1) != 0)));
-    if (norms_host) norms_host[i] = info.norm;
-    if (spec_host) spec_host[i] = 0;
+    if (spec_host) spec_host[i] = accepted ? 1 : 0;
   }
   return TNB_OK;
+}
+
+template <typename T>
+inline int ttsvd_batch_impl(void* workspace, size_t per_tensor_bytes, int inflight, const T* const* data, int batch,
+                            const SweepDims& d, const int32_t* rmax, double eps, uint32_t flags, T* const* cores,
+                            int32_t* ranks_host, double* norms_host, int32_t* spec_host, cudaStream_t st) {
+  const int N = d.N;
+  char* ws = static_cast<char*>(workspace);
+  auto ranks = [&](int i) { return ranks_host + (size_t)i * (N + 1); };
+  auto one = [&](Arena& ar, int i, SweepInfo* info) {
+    TNB_TRY((ttsvd_impl<T, Arena>(ar, false, data[i], d, rmax, eps, flags, cores[i], ranks(i), info, st)));
+    if (norms_host) norms_host[i] = info->norm;
+    return TNB_OK;
+  };
+  auto enqueue = [&](cudaStream_t* streams, int inflight, SpecHostBack* hbs) {
+    const uint32_t bflags = (flags | TNB_FLAG_CONCURRENT) & ~TNB_FLAG_PROFILE;
+    int rc = TNB_OK;
+    for (int g0 = 0; g0 < batch && rc == TNB_OK; g0 += inflight) {
+      const int g = std::min(inflight, batch - g0);
+      std::vector<Arena> arenas;
+      arenas.reserve(g);
+      std::vector<SpecRun<T, Arena>> runs(g);
+      for (int s = 0; s < g; ++s) arenas.emplace_back(ws + (size_t)s * per_tensor_bytes, per_tensor_bytes);
+      for (int s = 0; s < g && rc == TNB_OK; ++s)
+        rc = spec_begin<T, Arena>(runs[s], arenas[s], false, data[g0 + s], d, eps, bflags, cores[g0 + s], nullptr, streams[s]);
+      // Enqueued step by step: all Gram kernels of a step, then the eigen stages of all tensors interleaved stage by
+      // stage, then every tensor's rank rule + projection.  The resident filter kernels are chained across the streams
+      // (cheb_filter.cuh), so this order keeps tensor A's Rayleigh-Ritz step in flight while tensor B's filter runs; it
+      // measured faster than enqueuing each tensor's whole eigen chain at once or a diagonal wavefront over the steps
+      // (profiles/r02_batch_schedule.md).
+      for (int mu = N - 1, t = 0; mu >= 1 && rc == TNB_OK; --mu, ++t) {
+        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase1<T, Arena>(runs[s], false, d, mu, t, false);
+        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2a<T, Arena>(runs[s], false);
+        for (int stage = 0; stage <= CD_MAX_STAGES && rc == TNB_OK; ++stage)
+          for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2s<T, Arena>(runs[s], false, stage);
+        for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_phase2b<T, Arena>(runs[s], false, d, rmax, mu, t, false);
+      }
+      for (int s = 0; s < g && rc == TNB_OK; ++s) rc = spec_end<T, Arena>(runs[s], d, hbs + g0 + s);
+    }
+    return rc;
+  };
+  auto accept = [&](int i, const SpecHostBack& hb) {
+    SweepInfo info;
+    spec_accept(hb, d, ranks(i), &info);
+    if (norms_host) norms_host[i] = info.norm;
+  };
+  // exact Gram matrices when the TF32 one was rejected (flag bit 0)
+  auto repeat = [&](Arena& ar, int i, int spec_flags) {
+    SweepInfo info;
+    TNB_TRY((ttsvd_sync_impl<T, Arena>(ar, false, data[i], d, rmax, eps, flags & ~TNB_FLAG_PROFILE, cores[i], ranks(i), &info,
+                                       st, (spec_flags & 1) != 0)));
+    if (norms_host) norms_host[i] = info.norm;
+    return TNB_OK;
+  };
+  const bool spec = batch > 0 && spec_eligible<T>(d, rmax, eps, flags, tc_allowed(flags, false));
+  return spec_batch(workspace, per_tensor_bytes, inflight, batch, spec, spec_host, st, one, enqueue, accept, repeat);
 }
 
 }  // namespace tnb

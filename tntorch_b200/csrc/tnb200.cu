@@ -33,6 +33,27 @@ inline int require_device() {
 }
 // headroom for rank-dependent re-planning between the sizing pass (rank caps) and the run (actual ranks)
 inline size_t with_slack(size_t bytes) { return bytes + bytes / 8 + (size_t)(4 << 20); }
+
+// Workspace of a batch call: one slice of `one` bytes per tensor in flight, up to TNB_BATCH_MAX_INFLIGHT
+// (measured on B200: 4 -> 171, 6 -> 172, 8 -> 175 GElements/s).
+inline size_t batch_workspace_bytes(size_t one, int batch, size_t* per_tensor_bytes) {
+  if (per_tensor_bytes) *per_tensor_bytes = one;
+  if (one == 0 || batch < 1) return 0;
+  return one * (size_t)std::min(batch, TNB_BATCH_MAX_INFLIGHT);
+}
+
+// Checks shared by the batch entry points once their dims are known (cores buffers of `need` elements, a workspace
+// slice of `one` bytes per tensor, 0 for an unsupported shape), and how many tensors the workspace holds in flight.
+inline int batch_inflight(const char* fn, int64_t cores_capacity, int64_t need, size_t one, size_t workspace_bytes,
+                          int* inflight) {
+  if (cores_capacity < need)
+    return fail(TNB_ERR_WORKSPACE, "%s: cores buffers hold %lld elements, need %lld", fn, (long long)cores_capacity,
+                (long long)need);
+  if (one == 0) return fail(TNB_ERR_UNSUPPORTED, "%s: unsupported shape", fn);
+  if (workspace_bytes < one) return fail(TNB_ERR_WORKSPACE, "%s: workspace %zu < %zu", fn, workspace_bytes, one);
+  *inflight = (int)std::min<size_t>(workspace_bytes / one, (size_t)TNB_BATCH_MAX_INFLIGHT);
+  return TNB_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -114,11 +135,7 @@ int tnb_ttsvd(int dtype, const void* data, int ndim, const int64_t* shape, const
 
 size_t tnb_ttsvd_batch_workspace_bytes(int dtype, int batch, int ndim, const int64_t* shape, const int32_t* rmax,
                                        uint32_t flags, size_t* per_tensor_bytes) {
-  const size_t one = tnb_ttsvd_workspace_bytes(dtype, ndim, shape, rmax, flags);
-  if (per_tensor_bytes) *per_tensor_bytes = one;
-  if (one == 0 || batch < 1) return 0;
-  const int inflight = batch < TNB_BATCH_MAX_INFLIGHT ? batch : TNB_BATCH_MAX_INFLIGHT;  // measured on B200: 4 -> 171, 6 -> 172, 8 -> 175 GElements/s
-  return one * (size_t)inflight;
+  return batch_workspace_bytes(tnb_ttsvd_workspace_bytes(dtype, ndim, shape, rmax, flags), batch, per_tensor_bytes);
 }
 
 int tnb_ttsvd_batch(int dtype, const void* const* data, int batch, int ndim, const int64_t* shape, const int32_t* rmax,
@@ -134,15 +151,11 @@ int tnb_ttsvd_batch(int dtype, const void* const* data, int batch, int ndim, con
       if (rmax[k] < 0) return fail(TNB_ERR_INVALID, "rmax[%d] must be >= 1 (or 0 for none)", k);
   SweepDims d;
   TNB_TRY(make_dims(ndim, shape, rmax, d));
-  if (cores_capacity < d.capacity)
-    return fail(TNB_ERR_WORKSPACE, "tnb_ttsvd_batch: cores buffers hold %lld elements, need %lld", (long long)cores_capacity,
-                (long long)d.capacity);
   for (int i = 0; i < batch; ++i)
     if (!data[i] || !cores[i]) return fail(TNB_ERR_INVALID, "tnb_ttsvd_batch: null tensor %d", i);
   const size_t one = tnb_ttsvd_workspace_bytes(dtype, ndim, shape, rmax, flags);
-  if (one == 0) return fail(TNB_ERR_UNSUPPORTED, "tnb_ttsvd_batch: unsupported shape");
-  if (workspace_bytes < one) return fail(TNB_ERR_WORKSPACE, "tnb_ttsvd_batch: workspace %zu < %zu", workspace_bytes, one);
-  const int inflight = (int)std::min<size_t>(workspace_bytes / one, (size_t)TNB_BATCH_MAX_INFLIGHT);
+  int inflight;
+  TNB_TRY(batch_inflight("tnb_ttsvd_batch", cores_capacity, d.capacity, one, workspace_bytes, &inflight));
   if (dtype == TNB_F32)
     return ttsvd_batch_impl<float>(workspace, one, inflight, reinterpret_cast<const float* const*>(data), batch, d, rmax, eps,
                                    flags, reinterpret_cast<float* const*>(cores), ranks_host, norms_host, speculative_host,
@@ -223,10 +236,7 @@ int tnb_tt_round(int dtype, const void* const* cores_in, int ndim, const int64_t
 
 size_t tnb_tt_round_batch_workspace_bytes(int dtype, int batch, int ndim, const int64_t* shape, const int32_t* ranks_in,
                                           const int32_t* rmax, size_t* per_tensor_bytes) {
-  const size_t one = tnb_tt_round_workspace_bytes(dtype, ndim, shape, ranks_in, rmax);
-  if (per_tensor_bytes) *per_tensor_bytes = one;
-  if (one == 0 || batch < 1) return 0;
-  return one * (size_t)(batch < TNB_BATCH_MAX_INFLIGHT ? batch : TNB_BATCH_MAX_INFLIGHT);
+  return batch_workspace_bytes(tnb_tt_round_workspace_bytes(dtype, ndim, shape, ranks_in, rmax), batch, per_tensor_bytes);
 }
 
 int tnb_tt_round_batch(int dtype, const void* const* cores_in, int batch, int ndim, const int64_t* shape,
@@ -239,11 +249,9 @@ int tnb_tt_round_batch(int dtype, const void* const* cores_in, int batch, int nd
     return fail(TNB_ERR_INVALID, "tnb_tt_round_batch: null argument");
   RoundDims d;
   TNB_TRY(make_round_dims(ndim, shape, ranks_in, rmax, d));
-  if (cores_capacity < d.capacity) return fail(TNB_ERR_WORKSPACE, "tnb_tt_round_batch: cores buffers too small");
   const size_t one = tnb_tt_round_workspace_bytes(dtype, ndim, shape, ranks_in, rmax);
-  if (one == 0) return fail(TNB_ERR_UNSUPPORTED, "tnb_tt_round_batch: unsupported shape");
-  if (workspace_bytes < one) return fail(TNB_ERR_WORKSPACE, "tnb_tt_round_batch: workspace %zu < %zu", workspace_bytes, one);
-  const int inflight = (int)std::min<size_t>(workspace_bytes / one, (size_t)TNB_BATCH_MAX_INFLIGHT);
+  int inflight;
+  TNB_TRY(batch_inflight("tnb_tt_round_batch", cores_capacity, d.capacity, one, workspace_bytes, &inflight));
   if (dtype == TNB_F32)
     return tt_round_batch_impl<float>(workspace, one, inflight, reinterpret_cast<const float* const*>(cores_in), batch, d, rmax,
                                       eps, flags, reinterpret_cast<float* const*>(cores_out), ranks_host, speculative_host,

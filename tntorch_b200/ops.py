@@ -273,8 +273,9 @@ def ttsvd_batch(tensors, rmax=None, eps: float = 1e-14, batch_mode: bool = False
 
 
 # --------------------------------------------------------------------------------------
-def tt_round(cores: Sequence[torch.Tensor], eps: float = 1e-14, rmax=None, batch_mode: bool = False):
-    """Tensor.round_tt on device cores (tensor.py:2008-2083). Returns new cores."""
+def tt_round(cores: Sequence[torch.Tensor], eps: float = 1e-14, rmax=None, batch_mode: bool = False, speculate: bool = True):
+    """Tensor.round_tt on device cores (tensor.py:2008-2083). Returns new cores.  speculate=False takes the host-driven
+    sweeps even where the single-synchronisation path could run (TNB_FLAG_NO_SPECULATE)."""
     N = len(cores)
     for c in cores:
         _require_cuda(c, "tt_round")
@@ -304,7 +305,7 @@ def tt_round(cores: Sequence[torch.Tensor], eps: float = 1e-14, rmax=None, batch
     out = torch.empty(int(cap), dtype=dt, device=dev)
     ranks = (C.c_int32 * (N + 1))()
     ptrs = (C.c_void_p * N)(*[c.data_ptr() for c in cores])
-    flags = _lib.FLAG_BATCH_MODE if batch_mode else 0
+    flags = (_lib.FLAG_BATCH_MODE if batch_mode else 0) | (0 if speculate else _lib.FLAG_NO_SPECULATE)
     with torch.cuda.device(dev):
         check(L.tnb_tt_round(code, ptrs, N, sh, rinc, rmc, float(eps), flags, _ptr(ws), ws.numel(), _ptr(out), cap, ranks,
                              _stream()))
